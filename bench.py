@@ -5,6 +5,7 @@
     python bench.py --model fcos ...                                   # DGFCOS dg (configs[2])
     python bench.py --exp non_dg ...                                   # mode 0 only (DGFRCNN.py:128)
     python bench.py --impl reference --gpus N --steps K --warmup W     # the reference's own code on the host CPU
+    python bench.py ... --dump-outputs DIR                             # also save the last timed step's results (.npy)
 
 A *step* is one pass of the reference's 8-training-step mode cycle (0,1,0,2,0,3,0,4 — DGFRCNN.py:125-199,
 DGFCOS.py:164-243; `non_dg`: eight mode-0 steps) over synthetic 3x800x1333 batches: 8*B images per GPU, optimizer
@@ -68,6 +69,8 @@ def parse():
                    help="keep FrozenBatchNorm2d as separate elementwise passes (default: folded into the conv, utils.py)")
     p.add_argument("--memory-format", default="channels_last", choices=["channels_last", "contiguous"],
                    help="memory format of the detector's convolutions / FPN features")
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="write what the last timed step computed to DIR/*.npy (see dump_outputs), to compare two builds")
     return p.parse_args()
 
 
@@ -172,6 +175,35 @@ def cycle_modes(exp):
     return CYCLE if exp == "dg" else (0,) * len(CYCLE)
 
 
+DUMP_PER_TENSOR = 1 << 15
+
+
+def dump_outputs(out_dir, model, losses):
+    """Writes what one timed step hands back to its caller, in float32:
+      losses.npy  the loss returned by each training step of the step, in schedule order
+      params.npy  every parameter after the step's last optimizer update, concatenated in named_parameters() order
+    A tensor of more than DUMP_PER_TENSOR elements contributes a fixed sample of them (positions drawn by a generator
+    seeded with the parameter's name), so that runs and builds are compared entry for entry (about 10 MB for either
+    model).  Gradients are left out: after a few cycles the nondeterministic order of GPU reductions has changed which
+    proposals survive NMS, and the last backward's gradients are mostly run-to-run noise (two runs of the same build,
+    --steps 3 --warmup 3 on one B200 at 1000 W: gradients 49 % apart in relative L2 norm, losses at most 0.6 %,
+    parameters 1e-5)."""
+    import zlib
+
+    import numpy as np
+    import torch
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    params = []
+    for name, p in model.named_parameters():
+        n = p.numel()
+        idx = (np.arange(n) if n <= DUMP_PER_TENSOR else
+               np.sort(np.random.default_rng(zlib.crc32(name.encode())).choice(n, DUMP_PER_TENSOR, replace=False)))
+        params.append(p.detach().flatten()[torch.from_numpy(idx).to(p.device)])
+    np.save(out / "losses.npy", torch.stack(losses).float().cpu().numpy())
+    np.save(out / "params.npy", torch.cat(params).float().cpu().numpy())
+
+
 # --------------------------------------------------------------------------------------------- CUDA arm
 class B200Run:
     """One model instance of this repo on the current device + the loops that time it."""
@@ -256,10 +288,9 @@ class B200Run:
         torch = self.torch
         n = len(self.modes)
         if not from_host:
-            last = None
-            for s in range(n):
-                last = self.train_step(self.resident[(s // 2) % 4])
-            return last
+            # detached: the losses outlive the cycle for dump_outputs, their autograd graphs do not
+            self.losses = [self.train_step(self.resident[(s // 2) % 4]).detach() for s in range(n)]
+            return self.losses[-1]
         # end to end: every step's inputs come from the host and every step's loss goes back to it.  The copy of step s+1
         # overlaps the compute of step s, and the loss of step s is read while step s+1 is queued (the host stays one step
         # ahead instead of draining the GPU after every step).
@@ -397,6 +428,8 @@ def run_b200(args):
     ms = run.timed(args.steps, False)
     torch.cuda.profiler.stop()
     launches = _lib.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, run.model, run.losses)
     final_loss = float(run.train_step(run.resident[0]).item())   # untimed: is the run still numerically sane?
     run.reset_schedule()
     ops.KernelTimer.enabled = False
