@@ -15,7 +15,7 @@ LIB_PATH = PKG_DIR / "libdgod_b200.so"
 MAX_LEVELS = 8
 MAX_CELL_ANCHORS = 16
 F32, BF16 = 0, 1
-ABI_VERSION = 2   # DGOD_ABI_VERSION of include/dgod_b200.h
+ABI_VERSION = 3   # DGOD_ABI_VERSION of include/dgod_b200.h
 
 vp, i32, i64, f32, f64, sz = C.c_void_p, C.c_int, C.c_int64, C.c_float, C.c_double, C.c_size_t
 
@@ -55,7 +55,7 @@ SIGNATURES = {
     "dgod_matcher_workspace_bytes": (sz, [i32]),
     "dgod_matcher": (i32, [vp, i32, i32, f64, f64, i32, vp, vp, sz, vp]),
     "dgod_iou_match_workspace_bytes": (sz, [i32, i32]),
-    "dgod_iou_match": (i32, [vp, vp, vp, i32, i32, vp, vp, i32, i32, f64, f64, i32,
+    "dgod_iou_match": (i32, [vp, vp, vp, i32, i32, vp, vp, vp, i32, i32, f64, f64, i32,
                              vp, vp, vp, vp, vp, vp, sz, vp]),
     "dgod_fcos_assign": (i32, [vp, i32, i32, i32, f64, vp, vp, vp, i32, vp, vp, vp, vp, i32, vp]),
     "dgod_fcos_loss_workspace_bytes": (sz, [C.c_longlong]),
@@ -63,6 +63,8 @@ SIGNATURES = {
     "dgod_fcos_loss_bwd": (i32, [vp, vp, vp, vp, vp, vp, i32, i32, i32, f32, vp, vp, vp, vp, vp, vp]),
     "dgod_fcos_candidates": (i32, [vp, vp, vp, vp, i32, i32, vp, i32, i32, vp, f32, i32, vp, vp, vp, vp, vp, vp]),
     "dgod_balanced_sample": (i32, [vp, i32, vp, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp]),
+    "dgod_sample_rois": (i32, [vp, vp, i32, vp, vp, i32, vp, vp, i32, i32, vp, vp, i32, vp, vp, i32, f32, f32, f32, f32,
+                               vp, vp, vp, vp]),
     "dgod_nms_workspace_bytes": (sz, [i32, i32, i32]),
     "dgod_nms_batched": (i32, [vp, vp, vp, vp, vp, i32, i32, i32, f64, i32, i32, vp, vp, vp, vp, sz, vp]),
     "dgod_rpn_workspace_bytes": (sz, [C.POINTER(RpnConfig)]),

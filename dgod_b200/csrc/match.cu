@@ -45,24 +45,56 @@ __global__ void __launch_bounds__(256) box_iou_kernel(const float* __restrict__ 
 }
 
 // ---------------------------------------------------------------------------- fused path
+// The candidate slots of one image in the three layouts of dgod_iou_match.  Slot n < nb gets its outputs at out0 + n;
+// it holds a box when n < nv: row b0 + n of `boxes` while n < n_prop, past that (padded layout) ground truth n - n_prop.
+struct ImageSlots {
+  int nb, nv, n_prop;
+  long long b0, out0;
+};
+
+__device__ __forceinline__ ImageSlots image_slots(int img, int n_gt, const int32_t* __restrict__ box_offsets,
+                                                  const int32_t* __restrict__ box_counts, int n_boxes, int n_slots) {
+  ImageSlots s;
+  if (box_offsets) {                       // ragged: image i owns boxes[box_offsets[i] .. box_offsets[i+1])
+    s.b0 = s.out0 = box_offsets[img];
+    s.nb = s.nv = s.n_prop = box_offsets[img + 1] - box_offsets[img];
+  } else if (box_counts) {                 // padded [n_img, n_boxes] rows, the image's ground truths appended
+    s.b0 = (long long)img * n_boxes;
+    s.out0 = (long long)img * n_slots;
+    s.n_prop = min(max(box_counts[img], 0), n_boxes);
+    s.nb = n_slots;
+    s.nv = min(s.n_prop + n_gt, n_slots);
+  } else {                                 // one set of boxes shared by every image
+    s.b0 = 0;
+    s.out0 = (long long)img * n_boxes;
+    s.nb = s.nv = s.n_prop = n_boxes;
+  }
+  return s;
+}
+
+__device__ __forceinline__ float4 slot_box(const ImageSlots& s, const float* __restrict__ boxes,
+                                           const float* __restrict__ gt_boxes, int g0, int n) {
+  return n < s.n_prop ? ld_box(boxes, s.b0 + n) : ld_box(gt_boxes, g0 + (n - s.n_prop));
+}
+
 // Pass 1 (allow_low_quality only): row maximum of the implicit IoU matrix per ground truth.
 __global__ void __launch_bounds__(kMatchThreads)
 iou_rowmax_kernel(const float* __restrict__ gt_boxes, const int32_t* __restrict__ gt_offsets,
                   const float* __restrict__ boxes, const int32_t* __restrict__ box_offsets,
-                  int n_shared, uint32_t* __restrict__ gt_max /* ordered keys, zero-initialised */) {
+                  const int32_t* __restrict__ box_counts, int n_boxes, int n_slots,
+                  uint32_t* __restrict__ gt_max /* ordered keys, zero-initialised */) {
   __shared__ GtTile tile;
   __shared__ uint32_t smax[kGtChunk];
   const int img = blockIdx.y;
   const int g0 = gt_offsets[img], g1 = gt_offsets[img + 1];
-  int b0 = 0, nb = n_shared;
-  if (box_offsets) { b0 = box_offsets[img]; nb = box_offsets[img + 1] - b0; }
+  const ImageSlots s = image_slots(img, g1 - g0, box_offsets, box_counts, n_boxes, n_slots);
   const int n = blockIdx.x * blockDim.x + threadIdx.x;
-  if (blockIdx.x * blockDim.x >= nb) return;  // whole block idle (uniform)
-  const bool active = n < nb;
+  if (blockIdx.x * blockDim.x >= s.nv) return;  // whole block idle (uniform)
+  const bool active = n < s.nv;
   float4 bx = make_float4(0, 0, 0, 0);
   float ba = 0.f;
   if (active) {
-    bx = ld_box(boxes, b0 + n);
+    bx = slot_box(s, boxes, gt_boxes, g0, n);
     ba = box_area_exact(bx.x, bx.y, bx.z, bx.w);
   }
   for (int c0 = g0; c0 < g1; c0 += kGtChunk) {
@@ -86,7 +118,8 @@ iou_rowmax_kernel(const float* __restrict__ gt_boxes, const int32_t* __restrict_
 __global__ void __launch_bounds__(kMatchThreads)
 iou_match_kernel(const float* __restrict__ gt_boxes, const int64_t* __restrict__ gt_labels,
                  const int32_t* __restrict__ gt_offsets, const float* __restrict__ boxes,
-                 const int32_t* __restrict__ box_offsets, int n_shared, float high, float low,
+                 const int32_t* __restrict__ box_offsets, const int32_t* __restrict__ box_counts, int n_boxes,
+                 int n_slots, float high, float low,
                  const uint32_t* __restrict__ gt_max /* NULL when !allow_low_quality */,
                  int64_t* __restrict__ matched_idx, float* __restrict__ labels_f32,
                  int64_t* __restrict__ labels_i64, int64_t* __restrict__ clamped_idx,
@@ -95,16 +128,14 @@ iou_match_kernel(const float* __restrict__ gt_boxes, const int64_t* __restrict__
   __shared__ uint32_t smax[kGtChunk];
   const int img = blockIdx.y;
   const int g0 = gt_offsets[img], g1 = gt_offsets[img + 1];
-  int b0 = 0, nb = n_shared;
-  long long out0 = (long long)img * n_shared;
-  if (box_offsets) { b0 = box_offsets[img]; nb = box_offsets[img + 1] - b0; out0 = b0; }
+  const ImageSlots s = image_slots(img, g1 - g0, box_offsets, box_counts, n_boxes, n_slots);
   const int n = blockIdx.x * blockDim.x + threadIdx.x;
-  if (blockIdx.x * blockDim.x >= nb) return;
-  const bool active = n < nb;
+  if (blockIdx.x * blockDim.x >= s.nb) return;
+  const bool active = n < s.nv;
   float4 bx = make_float4(0, 0, 0, 0);
   float ba = 0.f;
   if (active) {
-    bx = ld_box(boxes, b0 + n);
+    bx = slot_box(s, boxes, gt_boxes, g0, n);
     ba = box_area_exact(bx.x, bx.y, bx.z, bx.w);
   }
   float best = 0.f;
@@ -126,7 +157,16 @@ iou_match_kernel(const float* __restrict__ gt_boxes, const int64_t* __restrict__
       }
     }
   }
-  if (!active) return;
+  if (n >= s.nb) return;
+  const long long o = s.out0 + n;
+  if (!active) {                           // padded layout: a slot past the image's candidates is ignored
+    if (matched_idx) matched_idx[o] = -2;
+    if (clamped_idx) clamped_idx[o] = 0;
+    if (labels_f32) labels_f32[o] = -1.f;
+    if (labels_i64) labels_i64[o] = -1;
+    if (matched_boxes) reinterpret_cast<float4*>(matched_boxes)[o] = make_float4(0, 0, 0, 0);
+    return;
+  }
   long long idx;
   if (best_m < 0) {
     idx = -1;  // image without ground truth: everything is background
@@ -136,7 +176,6 @@ iou_match_kernel(const float* __restrict__ gt_boxes, const int64_t* __restrict__
     else if (best < high) idx = -2;                  // BETWEEN_THRESHOLDS (best >= low here)
     if (tie_with_rowmax) idx = best_m;               // set_low_quality_matches_
   }
-  const long long o = out0 + n;
   const long long cl = idx < 0 ? 0 : idx;
   if (matched_idx) matched_idx[o] = idx;
   if (clamped_idx) clamped_idx[o] = cl;
@@ -244,18 +283,20 @@ extern "C" size_t dgod_iou_match_workspace_bytes(int n_img, int total_gt) {
 
 extern "C" int dgod_iou_match(const float* gt_boxes, const int64_t* gt_labels,
                               const int32_t* gt_offsets, int n_img, int total_gt,
-                              const float* boxes, const int32_t* box_offsets, int n_boxes,
-                              int max_boxes_per_img, double high_threshold, double low_threshold,
+                              const float* boxes, const int32_t* box_offsets, const int32_t* box_counts,
+                              int n_boxes, int max_boxes_per_img, double high_threshold, double low_threshold,
                               int allow_low_quality, int64_t* matched_idx, float* labels_f32,
                               int64_t* labels_i64, int64_t* clamped_idx, float* matched_boxes,
                               void* workspace, size_t workspace_bytes, dgod_stream_t stream) {
   DGOD_REQUIRE(n_img >= 0 && total_gt >= 0 && n_boxes >= 0 && max_boxes_per_img >= 0,
                "dgod_iou_match: negative size");
   DGOD_REQUIRE(low_threshold <= high_threshold, "low_threshold should be <= high_threshold");
-  if (n_img == 0 || n_boxes == 0 || max_boxes_per_img == 0) return DGOD_OK;
-  DGOD_REQUIRE(gt_offsets && boxes, "dgod_iou_match: null pointer");
+  DGOD_REQUIRE(!(box_offsets && box_counts), "dgod_iou_match: box_offsets and box_counts are exclusive");
+  if (n_img == 0 || max_boxes_per_img == 0 || (n_boxes == 0 && !box_counts)) return DGOD_OK;
+  DGOD_REQUIRE(gt_offsets && (boxes || n_boxes == 0), "dgod_iou_match: null pointer");
   DGOD_REQUIRE(total_gt == 0 || gt_boxes, "dgod_iou_match: gt_boxes is null");
-  if (!box_offsets) max_boxes_per_img = n_boxes;
+  DGOD_REQUIRE(!box_counts || max_boxes_per_img >= n_boxes, "dgod_iou_match: fewer slots than padded boxes");
+  if (!box_offsets && !box_counts) max_boxes_per_img = n_boxes;
   cudaStream_t st = (cudaStream_t)stream;
   dim3 grid(cdiv(max_boxes_per_img, kMatchThreads), n_img);
   uint32_t* gt_max = nullptr;
@@ -267,13 +308,13 @@ extern "C" int dgod_iou_match(const float* gt_boxes, const int64_t* gt_labels,
     gt_max = (uint32_t*)workspace;
     DGOD_CUDA(cudaMemsetAsync(gt_max, 0, (size_t)total_gt * sizeof(uint32_t), st));
     iou_rowmax_kernel<<<grid, kMatchThreads, 0, st>>>(gt_boxes, gt_offsets, boxes, box_offsets,
-                                                      n_boxes, gt_max);
+                                                      box_counts, n_boxes, max_boxes_per_img, gt_max);
     DGOD_LAUNCHED();
   }
   iou_match_kernel<<<grid, kMatchThreads, 0, st>>>(
-      gt_boxes, gt_labels, gt_offsets, boxes, box_offsets, n_boxes, (float)high_threshold,
-      (float)low_threshold, gt_max, matched_idx, labels_f32, labels_i64, clamped_idx,
-      matched_boxes);
+      gt_boxes, gt_labels, gt_offsets, boxes, box_offsets, box_counts, n_boxes, max_boxes_per_img,
+      (float)high_threshold, (float)low_threshold, gt_max, matched_idx, labels_f32, labels_i64,
+      clamped_idx, matched_boxes);
   DGOD_LAUNCHED();
   return DGOD_OK;
 }

@@ -254,6 +254,87 @@ balanced_sample_kernel(const L* __restrict__ labels, const float* __restrict__ k
   cluster.sync();                                          // no CTA leaves while its shared memory may still be read
 }
 
+// ---- sampled RoIs of the RoI heads (TV roi_heads.py:615-678 from the sampler's output on): one CTA per image
+constexpr int kRoiThreads = 512;
+constexpr int kRoiMaxList = 1024;        // sampler capacity per class (and batch_size_per_image) handled per image
+
+// number of entries of the ascending list a[0..n) below v
+__device__ __forceinline__ int count_below(const int* a, int n, int v) {
+  int lo = 0, hi = n;
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (a[mid] < v) lo = mid + 1; else hi = mid;
+  }
+  return lo;
+}
+
+// BoxCoder.encode_single (TV _utils.py:75-119) in the order of the torch composition (one rounding per operation)
+__device__ __forceinline__ float4 encode_box(float4 gt, float4 p, float wx, float wy, float ww, float wh) {
+  const float ex_w = __fsub_rn(p.z, p.x), ex_h = __fsub_rn(p.w, p.y);
+  const float ex_cx = __fadd_rn(p.x, __fmul_rn(0.5f, ex_w)), ex_cy = __fadd_rn(p.y, __fmul_rn(0.5f, ex_h));
+  const float gt_w = __fsub_rn(gt.z, gt.x), gt_h = __fsub_rn(gt.w, gt.y);
+  const float gt_cx = __fadd_rn(gt.x, __fmul_rn(0.5f, gt_w)), gt_cy = __fadd_rn(gt.y, __fmul_rn(0.5f, gt_h));
+  return make_float4(__fdiv_rn(__fmul_rn(wx, __fsub_rn(gt_cx, ex_cx)), ex_w),
+                     __fdiv_rn(__fmul_rn(wy, __fsub_rn(gt_cy, ex_cy)), ex_h),
+                     __fmul_rn(ww, logf(__fdiv_rn(gt_w, ex_w))), __fmul_rn(wh, logf(__fdiv_rn(gt_h, ex_h))));
+}
+
+__global__ void __launch_bounds__(kRoiThreads)
+sample_rois_kernel(const int64_t* __restrict__ pos_idx, const uint8_t* __restrict__ pos_valid, int cap_pos,
+                   const int64_t* __restrict__ neg_idx, const uint8_t* __restrict__ neg_valid, int cap_neg,
+                   const int64_t* __restrict__ labels, const int64_t* __restrict__ clamped_idx, int n_slots,
+                   const float* __restrict__ boxes, const int32_t* __restrict__ box_counts, int n_boxes,
+                   const float* __restrict__ gt_boxes, const int32_t* __restrict__ gt_offsets, int batch_size,
+                   float wx, float wy, float ww, float wh, float* __restrict__ s_props, int64_t* __restrict__ s_labels,
+                   float* __restrict__ reg_targets) {
+  __shared__ int pos[kRoiMaxList], neg[kRoiMaxList], sel[kRoiMaxList];
+  __shared__ int n_pos, n_neg;
+  const int img = blockIdx.x, tid = threadIdx.x;
+  pos_idx += (size_t)img * cap_pos; pos_valid += (size_t)img * cap_pos;
+  neg_idx += (size_t)img * cap_neg; neg_valid += (size_t)img * cap_neg;
+  if (tid == 0) n_pos = n_neg = 0;
+  __syncthreads();
+  // the sampler's lists are ascending with the valid entries first
+  for (int i = tid; i < cap_pos; i += kRoiThreads) {
+    pos[i] = (int)pos_idx[i];
+    if (pos_valid[i]) atomicAdd(&n_pos, 1);
+  }
+  for (int i = tid; i < cap_neg; i += kRoiThreads) {
+    neg[i] = (int)neg_idx[i];
+    if (neg_valid[i]) atomicAdd(&n_neg, 1);
+  }
+  __syncthreads();
+  // merge of the two (disjoint) ascending lists = torch.sort of their concatenation (roi_heads.py:620 torch.where order)
+  const int np = n_pos, nn = n_neg, n_sel = min(np + nn, batch_size);
+  for (int i = tid; i < np; i += kRoiThreads) {
+    const int r = i + count_below(neg, nn, pos[i]);
+    if (r < batch_size) sel[r] = pos[i];
+  }
+  for (int i = tid; i < nn; i += kRoiThreads) {
+    const int r = i + count_below(pos, np, neg[i]);
+    if (r < batch_size) sel[r] = neg[i];
+  }
+  __syncthreads();
+  const int g0 = gt_offsets[img], n_gt = gt_offsets[img + 1] - g0;
+  const int n_prop = min(max(box_counts[img], 0), n_boxes);
+  const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int s = tid; s < batch_size; s += kRoiThreads) {
+    const size_t o = (size_t)img * batch_size + s;
+    float4 box = zero, gt = n_gt > 0 ? ld_box(gt_boxes, g0) : zero, enc_box = make_float4(0.f, 0.f, 1.f, 1.f);
+    long long lab = -100;                  // an empty slot: cross_entropy's ignore_index, a zero box
+    if (s < n_sel) {
+      const int c = sel[s];
+      box = enc_box = c < n_prop ? ld_box(boxes, (long long)img * n_boxes + c) : ld_box(gt_boxes, g0 + (c - n_prop));
+      lab = labels[(size_t)img * n_slots + c];
+      if (n_gt > 0) gt = ld_box(gt_boxes, g0 + clamped_idx[(size_t)img * n_slots + c]);
+    }
+    reinterpret_cast<float4*>(s_props)[o] = box;
+    s_labels[o] = lab;
+    // empty slots encode against (0,0,1,1) so that log() stays finite
+    reinterpret_cast<float4*>(reg_targets)[o] = encode_box(gt, enc_box, wx, wy, ww, wh);
+  }
+}
+
 }  // namespace dgod
 
 using namespace dgod;
@@ -274,6 +355,28 @@ extern "C" int dgod_balanced_sample(const void* labels, int labels_are_int64, co
     balanced_sample_kernel<float><<<n_img * kSampCluster, kSampThreads, 0, (cudaStream_t)stream>>>(
         (const float*)labels, keys, n, num_pos, batch_size_per_image, cap_pos, cap_neg, pos_idx, pos_valid, neg_idx, neg_valid,
         counts);
+  DGOD_LAUNCHED();
+  return DGOD_OK;
+}
+
+extern "C" int dgod_sample_rois(const int64_t* pos_idx, const uint8_t* pos_valid, int cap_pos, const int64_t* neg_idx,
+                                const uint8_t* neg_valid, int cap_neg, const int64_t* labels, const int64_t* clamped_idx,
+                                int n_img, int n_slots, const float* boxes, const int32_t* box_counts, int n_boxes,
+                                const float* gt_boxes, const int32_t* gt_offsets, int batch_size_per_image, float wx,
+                                float wy, float ww, float wh, float* s_props, int64_t* s_labels, float* reg_targets,
+                                dgod_stream_t stream) {
+  DGOD_REQUIRE(n_img >= 0 && n_slots >= 0 && n_boxes >= 0 && cap_pos >= 0 && cap_neg >= 0 && batch_size_per_image >= 0,
+               "dgod_sample_rois: negative size");
+  DGOD_REQUIRE(cap_pos <= kRoiMaxList && cap_neg <= kRoiMaxList && batch_size_per_image <= kRoiMaxList,
+               "dgod_sample_rois: more than 1024 sampled RoIs per image");
+  if (n_img == 0 || batch_size_per_image == 0) return DGOD_OK;
+  DGOD_REQUIRE((cap_pos == 0 || (pos_idx && pos_valid)) && (cap_neg == 0 || (neg_idx && neg_valid)) && labels &&
+                   clamped_idx && (boxes || n_boxes == 0) && box_counts && gt_offsets && s_props && s_labels &&
+                   reg_targets,
+               "dgod_sample_rois: null pointer");
+  sample_rois_kernel<<<n_img, kRoiThreads, 0, (cudaStream_t)stream>>>(
+      pos_idx, pos_valid, cap_pos, neg_idx, neg_valid, cap_neg, labels, clamped_idx, n_slots, boxes, box_counts, n_boxes,
+      gt_boxes, gt_offsets, batch_size_per_image, wx, wy, ww, wh, s_props, s_labels, reg_targets);
   DGOD_LAUNCHED();
   return DGOD_OK;
 }

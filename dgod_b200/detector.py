@@ -14,8 +14,9 @@ Module and parameter names follow the reference so its checkpoints load unchange
 roi_heads.box_predictor.cls_score/bbox_pred.
 
 The positive/negative samplers (TV models/detection/_utils.py:11-71) draw the same uniform
-subsets as upstream but with fixed output shapes (masks instead of `torch.where`), so a training
-step needs a single device->host read (the proposal counts).
+subsets as upstream but with fixed output shapes (masks instead of `torch.where`), and the RoI heads
+take the RPN's proposals padded with their counts on the device, so a training step reads nothing
+back to the host.
 """
 from __future__ import annotations
 
@@ -217,52 +218,34 @@ class RoIHeads(nn.Module):
         self.weights = tuple(bbox_reg_weights or (10.0, 10.0, 5.0, 5.0))
         self.score_thresh, self.nms_thresh, self.detections_per_img = score_thresh, nms_thresh, detections_per_img
 
-    def select_training_samples(self, proposals: List[Tensor], targets, sampler_keys=None):
+    def select_training_samples(self, proposals, targets, sampler_keys=None):
         """TV models/detection/roi_heads.py:642-678 with exactly batch_size_per_image rows per
-        image (what fasterrcnn.py:211-212 and DGFRCNN.py:152-153 assume)."""
-        gt_boxes = [t["boxes"].to(proposals[0].dtype) for t in targets]
-        gt_labels = [t["labels"] for t in targets]
-        proposals = [torch.cat((p, g)) for p, g in zip(proposals, gt_boxes)]              # add_gt_proposals
-        sizes = [p.shape[0] for p in proposals]
-        m = ops.match_boxes(gt_boxes, proposals, self.fg_iou_thresh, self.bg_iou_thresh, False,
-                            gt_labels=gt_labels, want=("labels_i64", "clamped_idx"))
-        B, N = len(proposals), max(sizes)
-        S = self.batch_size_per_image
-        dev = proposals[0].device
-        if min(sizes) == N:                                                               # common case: no padding
-            labels = m["labels_i64"].view(B, N)
-            idxs = m["clamped_idx"].view(B, N)
-            props = torch.stack(proposals)
+        image (what fasterrcnn.py:211-212 and DGFRCNN.py:152-153 assume).
+
+        `proposals` is the RPN's padded output (boxes [B,cap,4], device counts [B]) or a list of per-image [n_i,4]
+        boxes.  The candidates of image i are its proposals followed by its ground truths (add_gt_proposals), in slots
+        [0, N) with N = cap + the largest ground-truth count (known from the shapes), unused slots ignored; matcher,
+        sampler and the sample epilogue all read the counts on the device, so no step waits on the host.  Returns
+        (s_props [B,S,4], s_labels int64 [B,S], reg_targets [B,S,4]).  An image with fewer than S candidates leaves
+        slots empty: the reference would mis-split its batch there (fasterrcnn.py:211-212 hard-codes 512 rows per
+        image); this mirror keeps the [B, S] shape DGFRCNN.py:152-153 relies on and marks the empty slots with label
+        -100 (cross_entropy's ignore_index, also inside the DG heads) and a zero box, excluded from both loss
+        denominators."""
+        if isinstance(proposals, tuple):
+            boxes, counts = proposals
         else:
-            labels = torch.full((B, N), -1, dtype=torch.int64, device=dev)
-            idxs = torch.zeros((B, N), dtype=torch.int64, device=dev)
-            props = torch.zeros((B, N, 4), dtype=proposals[0].dtype, device=dev)
-            for i, (l, c, p) in enumerate(zip(m["labels_i64"].split(sizes), m["clamped_idx"].split(sizes), proposals)):
-                labels[i, :sizes[i]], idxs[i, :sizes[i]], props[i, :sizes[i]] = l, c, p
+            boxes = torch.nn.utils.rnn.pad_sequence(list(proposals), batch_first=True)
+            counts = ops.device_constant(tuple(p.shape[0] for p in proposals), torch.int32, boxes.device)
+        gt_boxes = [t["boxes"].to(boxes.dtype) for t in targets]
+        m = ops.match_boxes(gt_boxes, (boxes, counts), self.fg_iou_thresh, self.bg_iou_thresh, False,
+                            gt_labels=[t["labels"] for t in targets], want=("labels_i64", "clamped_idx"))
+        labels = m["labels_i64"]
+        B, N = labels.shape
+        if sampler_keys is not None and sampler_keys.shape[1] < N:   # the padding slots are never picked (label -1)
+            sampler_keys = F.pad(sampler_keys, (0, N - sampler_keys.shape[1]), value=1.0)
         pos_idx, pos_valid, neg_idx, neg_valid = self.sampler(labels, sampler_keys)
-        chosen = torch.cat([torch.where(pos_valid, pos_idx, torch.full_like(pos_idx, N)),
-                            torch.where(neg_valid, neg_idx, torch.full_like(neg_idx, N))], dim=1)
-        if chosen.shape[1] < S:                                # fewer candidates than slots: pad with the sentinel
-            chosen = torch.cat([chosen, torch.full((B, S - chosen.shape[1]), N, dtype=chosen.dtype, device=dev)], dim=1)
-        sel = torch.sort(chosen, dim=1).values[:, :S]          # ascending index like torch.where (roi_heads.py:620)
-        # An image with fewer than S candidates (positives + negatives) leaves slots empty.  The reference would
-        # mis-split its batch there (fasterrcnn.py:211-212 hard-codes 512 rows per image); this mirror keeps the
-        # [B, S] shape DGFRCNN.py:152-153 relies on and marks the empty slots: label -100 (cross_entropy's
-        # ignore_index, also inside the DG heads), a zero box, excluded from both loss denominators.
-        slot_valid = sel < N
-        sel = sel.clamp(max=N - 1)
-        s_props = torch.gather(props, 1, sel[..., None].expand(-1, -1, 4)) * slot_valid[..., None]
-        s_labels = torch.where(slot_valid, torch.gather(labels, 1, sel), torch.full_like(sel, -100))
-        s_idxs = torch.gather(idxs, 1, sel) * slot_valid
-        max_gt = max([g.shape[0] for g in gt_boxes] + [1])
-        gt_pad = torch.zeros((B, max_gt, 4), dtype=props.dtype, device=dev)
-        for i, g in enumerate(gt_boxes):
-            gt_pad[i, :g.shape[0]] = g
-        matched_gt = torch.gather(gt_pad, 1, s_idxs[..., None].expand(-1, -1, 4))
-        safe = s_props.clone()
-        safe[..., 2:] += (~slot_valid)[..., None]              # empty slots encode against the box (0,0,1,1): log() stays finite
-        reg_targets = encode_boxes(matched_gt, safe, self.weights)
-        return s_props, s_idxs, s_labels, reg_targets
+        return ops.sample_rois(pos_idx, pos_valid, neg_idx, neg_valid, labels, m["clamped_idx"], boxes, counts,
+                               gt_boxes, self.batch_size_per_image, self.weights)
 
     def losses(self, class_logits, box_regression, labels, regression_targets):
         """fastrcnn_loss per image (fasterrcnn.py:198-236)."""
@@ -290,25 +273,26 @@ class RoIHeads(nn.Module):
         flat = keep + off[:, None]
         return (cb.view(-1, 4)[flat], cs.view(-1)[flat], cl.view(-1)[flat], info[:-1])
 
-    def forward(self, features, proposals: List[Tensor], image_sizes: List[Tuple[int, int]], targets=None,
-                sampler_keys=None):
+    def forward(self, features, proposals, image_sizes: List[Tuple[int, int]], targets=None, sampler_keys=None):
+        """`proposals`: in training the RPN's (boxes [B,cap,4], counts [B]) or a list of [n_i,4]; in eval a list."""
         dev = proposals[0].device
         sizes_t = ops.device_constant(tuple((float(h), float(w)) for h, w in image_sizes), torch.float32, dev)
-        labels = reg_targets = None
+        labels = reg_targets = label_list = None
         if self.training:
-            props, _, labels, reg_targets = self.select_training_samples(proposals, targets, sampler_keys)
-            prop_list = list(props.unbind(0))
+            props, labels, reg_targets = self.select_training_samples(proposals, targets, sampler_keys)
+            B, S = labels.shape
+            box_features = self.box_roi_pool(features, props, image_sizes)                # fasterrcnn.py:278
+            label_list = list(labels.unbind(0))
+            props, per_image = props.view(-1, 4), [S] * B
         else:
-            prop_list = proposals
-        box_features = self.box_roi_pool(features, prop_list, image_sizes)                # fasterrcnn.py:278
-        label_list = list(labels.unbind(0)) if labels is not None else None
+            box_features = self.box_roi_pool(features, proposals, image_sizes)
+            props, per_image = torch.cat(proposals), [p.shape[0] for p in proposals]
         box_features = self.box_head(box_features, label_list)                            # fasterrcnn.py:279
         class_logits, box_regression = self.box_predictor(box_features)
         losses = {}
         if self.training:
             losses = self.losses(class_logits, box_regression, labels, reg_targets)
-        per_image = [p.shape[0] for p in prop_list]
-        det = self.postprocess_detections(class_logits, box_regression, torch.cat(prop_list), per_image, sizes_t)
+        det = self.postprocess_detections(class_logits, box_regression, props, per_image, sizes_t)
         return det, losses, box_features, label_list
 
 
@@ -383,8 +367,10 @@ class FasterRCNN(nn.Module):
         keys = sampler_keys or {}
         (pb, ps, pc), rpn_losses = self.rpn(image_list.tensors.shape, image_list.image_sizes, features, targets,
                                             keys.get("rpn"))
-        counts = pc.tolist()                                   # the step's only device->host read
-        proposals = [pb[i, :c] for i, c in enumerate(counts)]
+        if self.training:
+            proposals = (pb, pc)                               # padded + device counts: training never reads them back
+        else:
+            proposals = [pb[i, :c] for i, c in enumerate(pc.tolist())]
         det, roi_losses, box_features, box_labels = self.roi_heads(features, proposals, image_list.image_sizes,
                                                                    targets, keys.get("roi"))
         self.last = {"features": features, "box_features": box_features, "box_labels": box_labels,

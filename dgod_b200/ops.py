@@ -286,19 +286,25 @@ class Matcher:
 
 @torch.library.custom_op("dgod_b200::iou_match", mutates_args=())
 def _iou_match_op(gt_boxes: Tensor, gt_labels: Optional[Tensor], gt_offsets: Tensor, boxes: Tensor,
-                  box_offsets: Optional[Tensor], max_boxes_per_img: int, high: float, low: float,
-                  allow_low_quality: bool, want: int) -> List[Tensor]:
+                  box_offsets: Optional[Tensor], box_counts: Optional[Tensor], max_boxes_per_img: int, high: float,
+                  low: float, allow_low_quality: bool, want: int) -> List[Tensor]:
     """want bitmask: 1 labels_f32, 2 labels_i64, 4 clamped_idx, 8 matched_boxes.
-    Returns [matched_idx, labels_f32, labels_i64, clamped_idx, matched_boxes] (empty if not wanted)."""
-    _need_cuda(gt_boxes, gt_labels, gt_offsets, boxes, box_offsets)
+    Returns [matched_idx, labels_f32, labels_i64, clamped_idx, matched_boxes] (empty if not wanted).
+    Layouts (include/dgod_b200.h): shared boxes [N,4]; ragged (box_offsets); padded boxes [B,cap,4] + box_counts [B]
+    with the ground truths appended, max_boxes_per_img slots per image."""
+    _need_cuda(gt_boxes, gt_labels, gt_offsets, boxes, box_offsets, box_counts)
     lib = _lib.load()
     dev = boxes.device
     gt_boxes, boxes = _f32c(gt_boxes), _f32c(boxes)
     n_img = gt_offsets.shape[0] - 1
     total_gt = gt_boxes.shape[0]
-    shared = box_offsets is None
-    n_boxes = boxes.shape[0]
-    shape = (n_img, n_boxes) if shared else (n_boxes,)
+    if box_counts is not None:
+        box_counts = box_counts.to(torch.int32).contiguous()
+        n_boxes = boxes.shape[1]
+        shape = (n_img, max_boxes_per_img)
+    else:
+        n_boxes = boxes.shape[0]
+        shape = (n_img, n_boxes) if box_offsets is None else (n_boxes,)
     idx = torch.empty(shape, dtype=torch.int64, device=dev)
     lf = torch.empty(shape if want & 1 else (0,), dtype=torch.float32, device=dev)
     li = torch.empty(shape if want & 2 else (0,), dtype=torch.int64, device=dev)
@@ -307,10 +313,10 @@ def _iou_match_op(gt_boxes: Tensor, gt_labels: Optional[Tensor], gt_offsets: Ten
     wsb = lib.dgod_iou_match_workspace_bytes(n_img, total_gt)
     ws = _ws(wsb, dev)
     n_out = idx.numel()
-    tok = KernelTimer.start("iou_match", 16 * total_gt + 16 * n_boxes + n_out * (8 + (4 if want & 1 else 0) + (8 if want & 2 else 0)
-                                                                                + (8 if want & 4 else 0) + (16 if want & 8 else 0)))
+    tok = KernelTimer.start("iou_match", 16 * total_gt + 16 * boxes.numel() // 4 + n_out * (8 + (4 if want & 1 else 0) + (8 if want & 2 else 0)
+                                                                                  + (8 if want & 4 else 0) + (16 if want & 8 else 0)))
     check(lib.dgod_iou_match(_p(gt_boxes), _p(gt_labels), _p(gt_offsets), n_img, total_gt, _p(boxes),
-                             _p(box_offsets), n_boxes, int(max_boxes_per_img), float(high), float(low),
+                             _p(box_offsets), _p(box_counts), n_boxes, int(max_boxes_per_img), float(high), float(low),
                              int(allow_low_quality), _p(idx), _p(lf) if want & 1 else None,
                              _p(li) if want & 2 else None, _p(ci) if want & 4 else None,
                              _p(mb) if want & 8 else None, _p(ws), wsb, _stream()))
@@ -319,13 +325,23 @@ def _iou_match_op(gt_boxes: Tensor, gt_labels: Optional[Tensor], gt_offsets: Ten
 
 
 @_iou_match_op.register_fake
-def _(gt_boxes, gt_labels, gt_offsets, boxes, box_offsets, max_boxes_per_img, high, low, allow_low_quality, want):
+def _(gt_boxes, gt_labels, gt_offsets, boxes, box_offsets, box_counts, max_boxes_per_img, high, low, allow_low_quality,
+      want):
     n_img = gt_offsets.shape[0] - 1
-    shape = (n_img, boxes.shape[0]) if box_offsets is None else (boxes.shape[0],)
+    if box_counts is not None:
+        shape = (n_img, max_boxes_per_img)
+    else:
+        shape = (n_img, boxes.shape[0]) if box_offsets is None else (boxes.shape[0],)
     e = lambda cond, s, dt: boxes.new_empty(s if cond else (0,), dtype=dt)
     return [boxes.new_empty(shape, dtype=torch.int64), e(want & 1, shape, torch.float32),
             e(want & 2, shape, torch.int64), e(want & 4, shape, torch.int64),
             e(want & 8, shape + (4,), torch.float32)]
+
+
+def _gt_batch(gt_boxes: Sequence[Tensor], dev) -> Tuple[Tensor, Tensor]:
+    """Ground truths of a batch concatenated [sum M_i, 4] fp32 + int32 offsets [B+1] (from the shapes)."""
+    gt_cat = torch.cat([g.reshape(-1, 4).float() for g in gt_boxes]) if len(gt_boxes) else torch.zeros((0, 4), device=dev)
+    return gt_cat, _offsets([g.shape[0] for g in gt_boxes], dev)
 
 
 def match_boxes(gt_boxes: Sequence[Tensor], boxes, high_threshold: float, low_threshold: float,
@@ -333,18 +349,25 @@ def match_boxes(gt_boxes: Sequence[Tensor], boxes, high_threshold: float, low_th
                 want=("labels_f32",)):
     """Fused box_iou + Matcher (+ label / matched-box gather) for a batch of images.
 
-    gt_boxes: list of [M_i,4].  boxes: one Tensor [N,4] shared by all images (RPN anchors; results
-    are [B,N]) or a list of [N_i,4] (proposals; results are concatenated [sum N_i]).
+    gt_boxes: list of [M_i,4].  boxes is one of
+      * one Tensor [N,4] shared by all images (RPN anchors): results are [B,N];
+      * a list of [N_i,4] (proposals): results are concatenated [sum N_i];
+      * a pair (padded [B,cap,4], device counts [B]) (RPN output): image i's candidates are its first counts[i] boxes
+        followed by its ground truths (add_gt_proposals without the copy) and results are [B, cap + max M_i], -1 labels in
+        the slots past count_i + M_i.  Nothing is read back to the host.
     Returns a dict with 'matched_idx' plus the requested 'labels_f32' (TV rpn.py:216-225),
     'labels_i64' / 'clamped_idx' (TV roi_heads.py:597-609), 'matched_boxes'."""
     dev = gt_boxes[0].device if len(gt_boxes) else boxes.device
-    gt_cat = torch.cat([g.reshape(-1, 4).float() for g in gt_boxes]) if len(gt_boxes) else torch.zeros((0, 4), device=dev)
+    gt_cat, gt_off = _gt_batch(gt_boxes, dev)
     gl_cat = None
     if gt_labels is not None:
         gl_cat = torch.cat([l.reshape(-1).to(torch.int64) for l in gt_labels]).contiguous()
-    gt_off = _offsets([g.shape[0] for g in gt_boxes], dev)
+    box_off = box_counts = None
     if isinstance(boxes, Tensor):
-        bx, box_off, max_n = boxes, None, boxes.shape[0]
+        bx, max_n = boxes, boxes.shape[0]
+    elif isinstance(boxes, tuple):
+        bx, box_counts = boxes
+        max_n = bx.shape[1] + max([g.shape[0] for g in gt_boxes], default=0)
     else:
         bx = torch.cat(list(boxes))
         box_off = _offsets([b.shape[0] for b in boxes], dev)
@@ -353,8 +376,9 @@ def match_boxes(gt_boxes: Sequence[Tensor], boxes, high_threshold: float, low_th
     mask = 0
     for w in want:
         mask |= bits[w]
-    idx, lf, li, ci, mb = _eager(_iou_match_op)(gt_cat, gl_cat, gt_off, bx, box_off, max_n, float(high_threshold),
-                                        float(low_threshold), bool(allow_low_quality_matches), mask)
+    idx, lf, li, ci, mb = _eager(_iou_match_op)(gt_cat, gl_cat, gt_off, bx, box_off, box_counts, max_n,
+                                                float(high_threshold), float(low_threshold),
+                                                bool(allow_low_quality_matches), mask)
     out = {"matched_idx": idx}
     for name, t in (("labels_f32", lf), ("labels_i64", li), ("clamped_idx", ci), ("matched_boxes", mb)):
         if name in want:
@@ -934,6 +958,37 @@ def balanced_sample(labels: Tensor, keys: Tensor, num_pos: int, batch_size_per_i
                                            _p(counts), _stream()))
     KernelTimer.stop(tok)
     return pos_idx, pos_valid, neg_idx, neg_valid, counts
+
+
+def sample_rois(pos_idx: Tensor, pos_valid: Tensor, neg_idx: Tensor, neg_valid: Tensor, labels: Tensor,
+                clamped_idx: Tensor, boxes: Tensor, counts: Tensor, gt_boxes: Sequence[Tensor],
+                batch_size_per_image: int, weights: Sequence[float]):
+    """The RoI heads' training samples (TV roi_heads.py:615-678 after the sampler) in one launch, no host
+    synchronisation.  `labels` / `clamped_idx` [B,N] are `match_boxes`' results over the padded candidates (boxes
+    [B,cap,4], counts [B], ground truths appended) and pos_* / neg_* what `balanced_sample` picked from them.  Returns
+    (s_props [B,S,4], s_labels int64 [B,S], reg_targets [B,S,4]) with S = batch_size_per_image: the picked candidates
+    in ascending index order, regression targets encoded with `weights`; slots left empty (fewer candidates than S) hold
+    a zero box, label -100 and a finite target."""
+    _need_cuda(pos_idx, pos_valid, neg_idx, neg_valid, labels, clamped_idx, boxes, counts)
+    B, N = labels.shape
+    S = int(batch_size_per_image)
+    dev = labels.device
+    gt_cat, gt_off = _gt_batch(gt_boxes, dev)
+    pos_idx, neg_idx = pos_idx.contiguous(), neg_idx.contiguous()
+    pos_valid, neg_valid = [(v if v.dtype in (torch.bool, torch.uint8) else v.to(torch.uint8)).contiguous()   # 1 byte each
+                            for v in (pos_valid, neg_valid)]
+    labels, clamped_idx = labels.contiguous(), clamped_idx.contiguous()
+    boxes, counts = _f32c(boxes), counts.to(torch.int32).contiguous()
+    s_props = torch.empty((B, S, 4), dtype=torch.float32, device=dev)
+    s_labels = torch.empty((B, S), dtype=torch.int64, device=dev)
+    reg_targets = torch.empty((B, S, 4), dtype=torch.float32, device=dev)
+    tok = KernelTimer.start("sample_rois", B * (pos_idx.shape[1] + neg_idx.shape[1]) * 9 + B * S * (2 * 16 + 16 + 8 + 8 + 16))
+    check(_lib.load().dgod_sample_rois(_p(pos_idx), _p(pos_valid), pos_idx.shape[1], _p(neg_idx), _p(neg_valid),
+                                       neg_idx.shape[1], _p(labels), _p(clamped_idx), B, N, _p(boxes), _p(counts),
+                                       boxes.shape[1], _p(gt_cat), _p(gt_off), S, *[float(w) for w in weights],
+                                       _p(s_props), _p(s_labels), _p(reg_targets), _stream()))
+    KernelTimer.stop(tok)
+    return s_props, s_labels, reg_targets
 
 
 # --------------------------------------------------------------------------------- RPN

@@ -8,7 +8,7 @@ TV ops/poolers.py:147-227 are fused into the kernel.
 """
 from __future__ import annotations
 
-from typing import Dict, List, Tuple
+from typing import Dict, List, Tuple, Union
 
 import torch
 from torch import Tensor
@@ -18,13 +18,22 @@ from . import ops
 
 
 class MultiScaleRoIAlign(tv_poolers.MultiScaleRoIAlign):
-    def forward(self, x: Dict[str, Tensor], boxes: List[Tensor], image_shapes: List[Tuple[int, int]]) -> Tensor:
+    def forward(self, x: Dict[str, Tensor], boxes: Union[List[Tensor], Tensor],
+                image_shapes: List[Tuple[int, int]]) -> Tensor:
+        """`boxes`: a list of per-image [n_i,4] tensors, or one [B,S,4] tensor (S boxes for every image)."""
         x_filtered = tv_poolers._filter_input(x, self.featmap_names)
         if self.scales is None or self.map_levels is None:
             self.scales, self.map_levels = tv_poolers._setup_scales(
                 x_filtered, image_shapes, self.canonical_scale, self.canonical_level)
-        rois = ops._convert_to_roi_format(boxes)
-        offsets = ops._offsets([b.shape[0] for b in boxes], rois.device) if len(boxes) == x_filtered[0].shape[0] else None
+        if isinstance(boxes, Tensor):
+            B, S = boxes.shape[:2]
+            ids = torch.arange(B, dtype=boxes.dtype, device=boxes.device).view(B, 1, 1).expand(B, S, 1)
+            rois = torch.cat((ids, boxes), dim=2).view(B * S, 5)
+            counts = [S] * B
+        else:
+            rois = ops._convert_to_roi_format(boxes)
+            counts = [b.shape[0] for b in boxes]
+        offsets = ops._offsets(counts, rois.device) if len(counts) == x_filtered[0].shape[0] else None
         m = self.map_levels
         return ops.multiscale_roi_align(
             x_filtered, rois, self.scales, tuple(self.output_size), self.sampling_ratio,

@@ -18,6 +18,7 @@
  *   dgod_fcos_loss_fwd/_bwd fcos.py:149-202 (focal + GIoU + centre-ness losses of FCOSHead.compute_loss)
  *   dgod_fcos_candidates    fcos.py:576-597 (FCOS.postprocess_detections up to the NMS: score, threshold, top-k, decode, clip)
  *   dgod_balanced_sample    TV models/detection/_utils.py:11-71 (BalancedPositiveNegativeSampler; fasterrcnn.py:119-123,272)
+ *   dgod_sample_rois        TV roi_heads.py:615-678 after the sampler (sampled boxes, labels, regression targets)
  *   dgod_nms_batched        TV ops/boxes.py:20-120 -> torchvision::nms (TV rpn.py:289,
  *                           TV roi_heads.py:728, fcos.py:608)
  *   dgod_rpn_proposals      fasterrcnn.py:174-182 -> TV _utils.py:162-224, TV rpn.py:231-297,
@@ -44,7 +45,7 @@ extern "C" {
 
 typedef void* dgod_stream_t; /* a cudaStream_t (0 = legacy default stream) */
 
-#define DGOD_ABI_VERSION 2
+#define DGOD_ABI_VERSION 3
 
 enum {
   DGOD_OK = 0,
@@ -85,9 +86,18 @@ int dgod_matcher(const float* quality /*device [m,n]*/, int m, int n,
 size_t dgod_iou_match_workspace_bytes(int n_img, int total_gt);
 /* Fused box_iou + Matcher + label gather for a batch of images; the [M,N] matrix is never
  * materialised.  gt boxes of image i are gt_boxes[gt_offsets[i] .. gt_offsets[i+1]).
- * Candidate boxes: if box_offsets == NULL all images share boxes[0..n_boxes) (RPN anchors) and
- * outputs are [n_img, n_boxes]; otherwise image i owns boxes[box_offsets[i]..box_offsets[i+1])
- * and outputs are [n_boxes] (n_boxes = total).  max_boxes_per_img bounds the per-image count.
+ * Candidate boxes, in one of three layouts:
+ *   shared   (box_offsets == NULL, box_counts == NULL): all images share boxes[0..n_boxes) (RPN
+ *            anchors); outputs are [n_img, n_boxes].
+ *   ragged   (box_offsets): image i owns boxes[box_offsets[i]..box_offsets[i+1]); outputs are
+ *            [n_boxes] (n_boxes = total).  max_boxes_per_img bounds the per-image count.
+ *   padded   (box_counts, device [n_img]): boxes is [n_img, n_boxes, 4] and image i's candidate j
+ *            is boxes[i, j] for j < box_counts[i], its ground truth j - box_counts[i] for
+ *            j < box_counts[i] + n_gt_i (TV roi_heads.py:574-578 add_gt_proposals, without the
+ *            copy), and an empty slot after that.  Outputs are [n_img, max_boxes_per_img]
+ *            (max_boxes_per_img >= n_boxes + the largest n_gt_i); an empty slot gets
+ *            matched_idx = -2, labels -1, clamped_idx 0, matched_boxes 0.  The counts stay on the
+ *            device: no host synchronisation.
  * An image with zero ground truths gets matched_idx = -1 everywhere (TV rpn.py:202-206,
  * roi_heads.py:586-592 semantics follow from the derived outputs below).
  * Optional outputs (NULL to skip):
@@ -99,7 +109,7 @@ int dgod_iou_match(const float* gt_boxes /*device [total_gt,4]*/,
                    const int64_t* gt_labels /*device [total_gt] or NULL*/,
                    const int32_t* gt_offsets /*device [n_img+1]*/, int n_img, int total_gt,
                    const float* boxes /*device*/, const int32_t* box_offsets /*device or NULL*/,
-                   int n_boxes, int max_boxes_per_img,
+                   const int32_t* box_counts /*device or NULL*/, int n_boxes, int max_boxes_per_img,
                    double high_threshold, double low_threshold, int allow_low_quality,
                    int64_t* matched_idx, float* labels_f32, int64_t* labels_i64,
                    int64_t* clamped_idx, float* matched_boxes,
@@ -168,6 +178,23 @@ int dgod_fcos_candidates(const float* cls_logits, const float* bbox_regression, 
 int dgod_balanced_sample(const void* labels, int labels_are_int64, const float* keys, int n_img, int n,
                          int num_pos, int batch_size_per_image, int64_t* pos_idx, uint8_t* pos_valid,
                          int64_t* neg_idx, uint8_t* neg_valid, int32_t* counts, dgod_stream_t stream);
+
+/* The RoI heads' sampled RoIs (TV roi_heads.py:615-678 after the sampler) for a batch in one launch, no host
+ * synchronisation.  Inputs: dgod_balanced_sample's pos_idx/pos_valid [n_img, cap_pos] and neg_idx/neg_valid
+ * [n_img, cap_neg] over the candidates of dgod_iou_match's padded layout (boxes [n_img, n_boxes, 4] with box_counts,
+ * ground truths appended), and that call's labels / clamped_idx [n_img, n_slots].  Per image the picked candidates in
+ * ascending index order (the union of the two ascending lists) fill batch_size_per_image slots:
+ *   s_props     [n_img, batch, 4] the candidate's box; 0 in an empty slot
+ *   s_labels    [n_img, batch]    int64, its label; -100 in an empty slot
+ *   reg_targets [n_img, batch, 4] BoxCoder(weights).encode of its matched ground truth (ground truth 0 of the image in an
+ *                                 empty slot, zeros for an image without any) against its box, or against (0,0,1,1)
+ *                                 in an empty slot; the arithmetic of the eager torch composition, op for op.
+ * cap_pos, cap_neg, batch_size_per_image <= 1024. */
+int dgod_sample_rois(const int64_t* pos_idx, const uint8_t* pos_valid, int cap_pos, const int64_t* neg_idx,
+                     const uint8_t* neg_valid, int cap_neg, const int64_t* labels, const int64_t* clamped_idx, int n_img,
+                     int n_slots, const float* boxes, const int32_t* box_counts, int n_boxes, const float* gt_boxes,
+                     const int32_t* gt_offsets, int batch_size_per_image, float wx, float wy, float ww, float wh,
+                     float* s_props, int64_t* s_labels, float* reg_targets, dgod_stream_t stream);
 
 /* ------------------------------------------------------------------ batched NMS */
 
