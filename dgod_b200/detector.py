@@ -31,6 +31,7 @@ from torchvision.models.detection.backbone_utils import resnet_fpn_backbone
 from torchvision.models.detection.faster_rcnn import FastRCNNPredictor
 from torchvision.models.detection.rpn import RPNHead
 from torchvision.models.detection.transform import GeneralizedRCNNTransform
+from torchvision.ops.feature_pyramid_network import FeaturePyramidNetwork
 
 from . import ops
 from .poolers import MultiScaleRoIAlign
@@ -335,6 +336,39 @@ class FusedTransform(GeneralizedRCNNTransform):
         return r
 
 
+# ------------------------------------------------------------------------------------ FPN
+class FusedFPN(FeaturePyramidNetwork):
+    """torchvision's FeaturePyramidNetwork (TV ops/feature_pyramid_network.py; fasterrcnn.py:317) whose top-down merge
+    runs natively on CUDA: the lateral 1x1 convs run without their bias, and `ops.fpn_top_down` adds the bias, the
+    nearest-upsampled coarser level and the lateral in one pass per level (one pass per level backward as well),
+    instead of a bias-add pass, a full-size upsampled copy and an add.  The coarsest lateral conv, the 3x3 layer
+    blocks and LastLevelMaxPool are the stock modules.  Same parameters, state-dict keys and results, bit for bit.  On
+    CPU it is torchvision's forward."""
+
+    def forward(self, x: Dict[str, Tensor]) -> Dict[str, Tensor]:
+        names, feats = list(x.keys()), list(x.values())
+        if not feats[-1].is_cuda:
+            return super().forward(x)
+        convs = [blk[0] for blk in self.inner_blocks]
+        top = self.inner_blocks[-1](feats[-1])
+        laterals = [conv._conv_forward(f, conv.weight, None) for conv, f in zip(convs[:-1], feats[:-1])]
+        inners = ops.fpn_top_down(laterals, [conv.bias for conv in convs[:-1]], top)
+        results = [blk(t) for blk, t in zip(self.layer_blocks, inners)]
+        if self.extra_blocks is not None:
+            results, names = self.extra_blocks(results, feats, names)
+        return OrderedDict(zip(names, results))
+
+
+def fuse_fpn(fpn: FeaturePyramidNetwork) -> None:
+    """Rebinds a stock FeaturePyramidNetwork without norm layers (each inner block a single biased Conv2d) to FusedFPN."""
+    if type(fpn) is not FeaturePyramidNetwork:
+        raise TypeError(f"fuse_fpn expects a torchvision FeaturePyramidNetwork, got {type(fpn).__name__}")
+    for blk in fpn.inner_blocks:
+        if len(blk) != 1 or type(blk[0]) is not nn.Conv2d or blk[0].bias is None:
+            raise TypeError("fuse_fpn: every inner block must be one Conv2d with a bias (no norm layer)")
+    fpn.__class__ = FusedFPN
+
+
 # ------------------------------------------------------------------------------------ detector
 class FasterRCNN(nn.Module):
     def __init__(self, num_classes: int = 9, min_size: int = 800, max_size: int = 1333,
@@ -343,6 +377,7 @@ class FasterRCNN(nn.Module):
         self.transform = FusedTransform(min_size, max_size, [0.0, 0.0, 0.0], [1.0, 1.0, 1.0])  # fasterrcnn.py:439-441
         self.backbone = resnet_fpn_backbone(backbone_name="resnet50", weights=None,
                                             trainable_layers=trainable_backbone_layers)   # fasterrcnn.py:317
+        fuse_fpn(self.backbone.fpn)
         oc = self.backbone.out_channels
         self.rpn = RegionProposalNetwork(oc, ((32,), (64,), (128,), (256,), (512,)), ((0.5, 1.0, 2.0),) * 5,
                                          batch_size_per_image=rpn_batch_size_per_image)

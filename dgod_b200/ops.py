@@ -1108,3 +1108,122 @@ def detect_candidates(class_logits: Tensor, box_regression: Tensor, proposals: T
                                              _p(cb), _p(cs), _p(cl), _p(cv), _stream()))
     KernelTimer.stop(tok)
     return cb, cs, cl, cv
+
+
+# --------------------------------------------------------------------------------- backbone boundary: FPN merge, stem
+def _map_layout(t: Tensor) -> Tuple[Tensor, bool]:
+    """(t as NHWC or NCHW dense fp32 memory, is NHWC).  A map whose two layouts coincide (1x1 pixels) runs as NCHW."""
+    if t.dtype != torch.float32 or t.dim() != 4:
+        raise RuntimeError(f"FPN / stem kernels take float32 [N, C, H, W] maps, got {t.dtype} {tuple(t.shape)}")
+    if t.is_contiguous():
+        return t, False
+    if t.is_contiguous(memory_format=torch.channels_last):
+        return t, True
+    return t.contiguous(), False
+
+
+def _like(t: Tensor, nhwc: bool) -> Tensor:
+    return t.contiguous(memory_format=torch.channels_last if nhwc else torch.contiguous_format)
+
+
+def fpn_merge(lat: Tensor, bias: Tensor, coarse: Tensor) -> Tensor:
+    """(lat + bias[c]) + F.interpolate(coarse, size=lat.shape[-2:], mode="nearest") in one pass, bit-exact
+    (dgod_fpn_merge_fwd); the result has lat's memory layout."""
+    _need_cuda(lat, bias, coarse)
+    lat, nhwc = _map_layout(lat)
+    coarse, bias = _like(coarse, nhwc), _f32c(bias)
+    n, c, h, w = lat.shape
+    if coarse.dtype != torch.float32 or coarse.shape[:2] != lat.shape[:2] or bias.shape != (c,):
+        raise RuntimeError(f"fpn_merge: lateral {tuple(lat.shape)}, bias {tuple(bias.shape)} and coarse "
+                           f"{tuple(coarse.shape)} float32 maps of one batch and channel count expected")
+    out = torch.empty_like(lat)
+    tok = KernelTimer.start("fpn_merge_fwd", 4 * (2 * lat.numel() + coarse.numel()))
+    check(_lib.load().dgod_fpn_merge_fwd(_p(lat), _p(bias), _p(coarse), _p(out), n, h, w, coarse.shape[2],
+                                         coarse.shape[3], c, int(nhwc), _stream()))
+    KernelTimer.stop(tok)
+    return out
+
+
+def fpn_merge_backward(g_fine: Optional[Tensor], g_lb: Optional[Tensor], coarse_shape) -> Optional[Tensor]:
+    """Gradient of a coarse FPN level: g_lb + upsample_nearest2d_backward(g_fine) in one pass, bit-exact with the ATen
+    backward followed by autograd's accumulation (dgod_fpn_merge_bwd).  None stands for a zero gradient."""
+    if g_fine is None:
+        return g_lb
+    _need_cuda(g_fine, g_lb)
+    g_fine, nhwc = _map_layout(g_fine)
+    n, c, h, w = g_fine.shape
+    if g_lb is not None:
+        g_lb = _like(g_lb, nhwc)
+        if g_lb.dtype != torch.float32 or tuple(g_lb.shape) != tuple(coarse_shape):
+            raise RuntimeError(f"fpn_merge_backward: gradient {tuple(g_lb.shape)} of the {tuple(coarse_shape)} level")
+        out = torch.empty_like(g_lb)
+    else:
+        out = torch.empty(tuple(coarse_shape), dtype=torch.float32, device=g_fine.device,
+                          memory_format=torch.channels_last if nhwc else torch.contiguous_format)
+    hc, wc = out.shape[2], out.shape[3]
+    tok = KernelTimer.start("fpn_merge_bwd", 4 * (g_fine.numel() + (2 if g_lb is not None else 1) * out.numel()))
+    check(_lib.load().dgod_fpn_merge_bwd(_p(g_fine), _p(g_lb), _p(out), n, h, w, hc, wc, c, int(nhwc), _stream()))
+    KernelTimer.stop(tok)
+    return out
+
+
+class _FpnTopDownFn(torch.autograd.Function):
+    """The FPN top-down chain (TV ops/feature_pyramid_network.py, FeaturePyramidNetwork.forward) from the bias-free lateral
+    conv outputs: last_inner[i] = (laterals[i] + biases[i]) + upsample(last_inner[i + 1]), last_inner[-1] = top.
+    Backward, finest level first: the gradient of level i is its own incoming gradient plus the 2x2 (in general: ATen's
+    nearest-backward window) sum of the gradient of level i - 1 — one launch per level, no upsample-backward pass and no
+    accumulation add.  A lateral's gradient is its level's gradient, the bias gradient its sum over (N, H, W) as the
+    convolution backward computes it."""
+
+    @staticmethod
+    def forward(ctx, top, *lats_and_biases):
+        k = len(lats_and_biases) // 2
+        lats, biases = lats_and_biases[:k], lats_and_biases[k:]
+        outs = [top]
+        for i in range(k - 1, -1, -1):
+            outs.insert(0, fpn_merge(lats[i], biases[i], outs[0]))
+        ctx.shapes = [tuple(t.shape) for t in outs]
+        ctx.set_materialize_grads(False)
+        return tuple(outs)
+
+    @staticmethod
+    def backward(ctx, *grads):
+        k = len(grads) - 1
+        g = grads[0]
+        g_lats, g_biases = [], []
+        for i in range(k):
+            g_lats.append(g)
+            g_biases.append(g.sum((0, 2, 3)) if g is not None and ctx.needs_input_grad[1 + k + i] else None)
+            g = fpn_merge_backward(g, grads[i + 1], ctx.shapes[i + 1])
+        return (g, *g_lats, *g_biases)
+
+
+def fpn_top_down(laterals: Sequence[Tensor], biases: Sequence[Tensor], top: Tensor) -> List[Tensor]:
+    """All K `last_inner` maps of the FPN top-down path, finest first: `laterals` are the K - 1 finer levels' 1x1 conv
+    outputs WITHOUT their bias, `biases` those convs' biases, `top` the coarsest level's conv output (bias included).
+    Bit-exact with torchvision's interpolate + add chain, forward and backward."""
+    if len(laterals) != len(biases):
+        raise ValueError("fpn_top_down: one bias per lateral map expected")
+    _need_cuda(top, *laterals, *biases)
+    return list(_FpnTopDownFn.apply(top, *laterals, *biases))
+
+
+def stem_pool(conv: Tensor, shift: Tensor) -> Tensor:
+    """max_pool2d(relu(conv + shift[c]), kernel 3, stride 2, padding 1) in one pass that reads the conv output once
+    (dgod_stem_pool_fwd), bit-exact with the three ATen ops including NaN propagation.  For a frozen stem only: it has
+    no backward, so nothing it gets may require grad.  The result has conv's memory layout."""
+    _need_cuda(conv, shift)
+    if conv.requires_grad or shift.requires_grad:
+        raise RuntimeError("stem_pool has no backward: the stem must be frozen and its input must not require grad")
+    conv, nhwc = _map_layout(conv)
+    shift = _f32c(shift)
+    n, c, h, w = conv.shape
+    if shift.shape != (c,):
+        raise RuntimeError(f"stem_pool: shift of shape ({c},) expected, got {tuple(shift.shape)}")
+    ho, wo = (h - 1) // 2 + 1, (w - 1) // 2 + 1
+    out = torch.empty((n, c, ho, wo), dtype=torch.float32, device=conv.device,
+                      memory_format=torch.channels_last if nhwc else torch.contiguous_format)
+    tok = KernelTimer.start("stem_pool", 4 * (conv.numel() + out.numel()))
+    check(_lib.load().dgod_stem_pool_fwd(_p(conv), _p(shift), _p(out), n, h, w, c, ho, wo, int(nhwc), _stream()))
+    KernelTimer.stop(tok)
+    return out

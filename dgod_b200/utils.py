@@ -46,16 +46,69 @@ class _FoldedConv2d(nn.Conv2d):
     product), the BN buffers stay in the BN module; only the two elementwise passes over the
     activation (x*s, +shift) and their backward disappear."""
 
-    def forward(self, x):
+    def _scale_shift(self):
         bn = self._folded_bn[0]
         scale = bn.weight * (bn.running_var + bn.eps).rsqrt()
-        shift = bn.bias - bn.running_mean * scale
+        return scale, bn.bias - bn.running_mean * scale
+
+    def forward(self, x):
+        scale, shift = self._scale_shift()
         return self._conv_forward(x, self.weight * scale.view(-1, 1, 1, 1), shift)
+
+
+class _FoldedStem(_FoldedConv2d):
+    """The folded conv1 of a frozen ResNet stem together with the ReLU and 3x3 / stride-2 max-pool behind it.  On CUDA:
+    the cuDNN convolution with w * s and no bias, then ONE native pass (ops.stem_pool) that adds the shift, applies the
+    ReLU and pools — it reads the conv output once and writes only the pooled map, where the stock ops make three
+    full-resolution passes (bias add, ReLU, pool).  The stem's `relu` and `maxpool` modules then pass through.  On CPU
+    it is the folded conv and the stock modules do the rest.  Only for a stem whose weights and input need no
+    gradient (trainable_layers <= 4): the fused pass has no backward."""
+
+    def forward(self, x):
+        if not x.is_cuda:
+            return super().forward(x)
+        from . import ops
+        scale, shift = self._scale_shift()
+        return ops.stem_pool(self._conv_forward(x, self.weight * scale.view(-1, 1, 1, 1), None), shift)
+
+
+class _StemReLU(nn.ReLU):
+    """A fused stem's ReLU: already applied by _FoldedStem on CUDA."""
+
+    def forward(self, x):
+        return x if x.is_cuda else super().forward(x)
+
+
+class _StemMaxPool(nn.MaxPool2d):
+    """A fused stem's max-pool: already applied by _FoldedStem on CUDA."""
+
+    def forward(self, x):
+        return x if x.is_cuda else super().forward(x)
+
+
+def _pair(v):
+    return tuple(v) if isinstance(v, (tuple, list)) else (v, v)
+
+
+def _fuse_frozen_stem(parent: nn.Module) -> None:
+    """Rebinds a ResNet stem (children conv1, bn1, relu, maxpool in that order, conv1 folded and frozen, the torchvision
+    pooling 3x3 / 2 / pad 1) to _FoldedStem + pass-through relu and maxpool."""
+    names = [k for k, _ in parent.named_children()][:4]
+    if names != ["conv1", "bn1", "relu", "maxpool"]:
+        return
+    conv, relu, pool = parent.conv1, parent.relu, parent.maxpool
+    if (type(conv) is _FoldedConv2d and not conv.weight.requires_grad and type(relu) is nn.ReLU
+            and type(pool) is nn.MaxPool2d and _pair(pool.kernel_size) == (3, 3) and _pair(pool.stride) == (2, 2)
+            and _pair(pool.padding) == (1, 1) and _pair(pool.dilation) == (1, 1) and not pool.ceil_mode):
+        conv.__class__ = _FoldedStem
+        relu.__class__ = _StemReLU
+        pool.__class__ = _StemMaxPool
 
 
 def fold_frozen_bn(module: nn.Module) -> int:
     """Rebinds every (Conv2d without bias, FrozenBatchNorm2d) sibling pair that torchvision's ResNet applies
     back to back (stem, Bottleneck conv1-3, downsample) so that the BN becomes the conv's epilogue.
+    A frozen stem additionally runs its shift, ReLU and max-pool as one native pass on CUDA (_FoldedStem).
     Call after `calibrate_frozen_bn`.  State-dict keys and parameters are unchanged.  Returns the
     number of folded pairs; `unfold_frozen_bn` restores the stock modules."""
     from torchvision.ops.misc import FrozenBatchNorm2d
@@ -75,13 +128,18 @@ def fold_frozen_bn(module: nn.Module) -> int:
                 child.__class__ = _Identity
                 n += 1
             prev = child
+        _fuse_frozen_stem(parent)
     return n
 
 
 def unfold_frozen_bn(module: nn.Module) -> None:
     from torchvision.ops.misc import FrozenBatchNorm2d
     for m in module.modules():
-        if isinstance(m, _FoldedConv2d):
+        if type(m) is _StemReLU:
+            m.__class__ = nn.ReLU
+        elif type(m) is _StemMaxPool:
+            m.__class__ = nn.MaxPool2d
+        elif isinstance(m, _FoldedConv2d):
             m._folded_bn[0].__class__ = FrozenBatchNorm2d
             del m._folded_bn
             m.__class__ = nn.Conv2d

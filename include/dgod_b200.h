@@ -32,6 +32,9 @@
  *   dgod_image_batch        TV models/detection/transform.py:102-255 (GeneralizedRCNNTransform: normalize, resize, batch;
  *                           fasterrcnn.py:439-441, fcos.py:483)
  *   dgod_nchw_to_nhwc       layout helper (no reference counterpart: torch's .contiguous(channels_last))
+ *   dgod_fpn_merge_fwd/_bwd TV ops/feature_pyramid_network.py FeaturePyramidNetwork.forward (lateral bias add, nearest
+ *                           upsample, add) and its autograd (upsample_nearest2d_backward + accumulation)
+ *   dgod_stem_pool_fwd      TV models/resnet.py ResNet._forward_impl: bn1 shift (folded), relu, maxpool of a frozen stem
  */
 #ifndef DGOD_B200_H_
 #define DGOD_B200_H_
@@ -45,7 +48,7 @@ extern "C" {
 
 typedef void* dgod_stream_t; /* a cudaStream_t (0 = legacy default stream) */
 
-#define DGOD_ABI_VERSION 3
+#define DGOD_ABI_VERSION 4
 
 enum {
   DGOD_OK = 0,
@@ -345,6 +348,27 @@ int dgod_image_batch_u8(const uint8_t* const* images, const int* in_h, const int
  * channels_last RoIAlign kernels. */
 int dgod_nchw_to_nhwc(const void* src, void* dst, int batch, int channels, int hw, int dtype,
                       dgod_stream_t stream);
+
+/* ------------------------------------------------------------------ backbone boundary: FPN top-down merge, stem */
+
+/* Maps are fp32 [n, c, h, w] in NCHW (channels_last = 0) or NHWC memory (channels_last = 1: c % 4 == 0 and every
+ * pointer 16-byte aligned).  All three are bit-exact with the ATen ops they replace.
+ *
+ * FPN merge: out = (lat + bias[c]) + nearest_upsample(coarse [n, c, hc, wc]) to [h, w], the two adds in that order, the
+ * source pixel as ATen's nearest mode computes it (min(floor(y * ((float)hc / h)), hc - 1), likewise x).  out may be
+ * the same buffer as lat. */
+int dgod_fpn_merge_fwd(const float* lat, const float* bias /*device [c]*/, const float* coarse, float* out, int n, int h,
+                       int w, int hc, int wc, int c, int channels_last, dgod_stream_t stream);
+/* Its backward for the coarse level: g_coarse = g_lb + (sum of g_fine [n, c, h, w] over the fine pixels of ATen's
+ * upsample_nearest2d_backward: rows [ceil(yc * s), ceil((yc + 1) * s)) clamped to h, s = (float)h / hc, likewise
+ * columns; summed row-major into a float starting at 0).  g_lb (the coarse level's other gradient) may be NULL (zero)
+ * and may be the same buffer as g_coarse. */
+int dgod_fpn_merge_bwd(const float* g_fine, const float* g_lb, float* g_coarse, int n, int h, int w, int hc, int wc,
+                       int c, int channels_last, dgod_stream_t stream);
+/* Frozen ResNet stem epilogue: out [n, c, ho, wo] = max_pool2d(relu(conv + shift[c]), 3, stride 2, pad 1) with
+ * ho = (h - 1) / 2 + 1, wo = (w - 1) / 2 + 1; NaN propagates as through clamp_min and max_pool2d.  No backward. */
+int dgod_stem_pool_fwd(const float* conv, const float* shift /*device [c]*/, float* out, int n, int h, int w, int c,
+                       int ho, int wo, int channels_last, dgod_stream_t stream);
 
 /* ------------------------------------------------------------------ gradient reversal */
 

@@ -14,7 +14,7 @@ torch.manual_seed(0)
 B = 8
 model = DGFRCNN(9, B, "dg", bench.REG_WEIGHTS, 2).to(dev).train().to(memory_format=torch.channels_last)
 res = [bench.to_device(b, dev) for b in bench.synthetic_batches(4, B, 2, 0)]
-bench.calibrate(model, res[0][0])
+bench.calibrate(model.detector, res[0][0])
 if "--eager" not in sys.argv:          # bench.py's default host-side setup: folded frozen BN + graphed backbone
     from dgod_b200.utils import fold_frozen_bn
     fold_frozen_bn(model.detector.backbone)
@@ -55,4 +55,4 @@ span = (max(e.time_range.end for e in kern) - min(e.time_range.start for e in ke
 print(f"GPU kernels over the 8-step cycle: {len(kern)} launches, {gpu_ms:.1f} ms busy in a {span:.1f} ms span "
       f"({100 * gpu_ms / span:.0f} % busy); dgod_b200 kernels {ours:.2f} ms")
 ka = prof.key_averages()
-print(prof.key_averages().table(sort_by="self_cuda_time_total", row_limit=40, max_name_column_width=70))
+print(prof.key_averages().table(sort_by="self_cuda_time_total", row_limit=-1, max_name_column_width=110))
