@@ -102,6 +102,18 @@ __device__ __forceinline__ float float_from_ordered(uint32_t k) {
   return __uint_as_float(u);
 }
 
+// ATen's relu_ on CUDA is clamp_min(v, 0) (TensorCompare.cu, launch_clamp_scalar): NaN passes through, everything else
+// is ::max(v, 0), i.e. fmaxf — the same instruction, so signed zeros come out as ATen's do.
+__device__ __forceinline__ float clamp_min0(float v) { return isnan(v) ? v : fmaxf(v, 0.f); }
+
+// Streaming passes over [rows x row_len] maps: rows go to the grid's y dimension (at most 65535, the kernels stride over
+// the rest), a row's elements to x in blocks of 256 threads.
+static inline dim3 row_grid(long long rows, int row_len) {
+  return dim3((unsigned)cdiv(row_len, 256), (unsigned)(rows < 65535 ? rows : 65535));
+}
+
+static inline bool aligned16(const void* p) { return ((uintptr_t)p & 15u) == 0; }
+
 __device__ __forceinline__ float4 ld_box(const float* p, long long i) {
   return __ldg(reinterpret_cast<const float4*>(p) + i);
 }

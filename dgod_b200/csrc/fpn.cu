@@ -31,8 +31,7 @@ __device__ __forceinline__ float4 add4(float4 a, float4 b) {
 
 // clamp_min(v, 0) with NaN passed through (TensorCompare.cu), then the max-pool's update rule (DilatedMaxPool2d.cu)
 __device__ __forceinline__ void relu_max(float& m, float v, float shift) {
-  float t = __fadd_rn(v, shift);
-  t = isnan(t) ? t : fmaxf(t, 0.f);
+  const float t = clamp_min0(__fadd_rn(v, shift));
   if (t > m || isnan(t)) m = t;
 }
 
@@ -142,13 +141,6 @@ stem_pool_kernel(const float* __restrict__ conv, const float* __restrict__ shift
     }
   }
 }
-
-// Rows go to the grid's y dimension (at most 65535, the kernels stride over the rest), a row's elements to x.
-static dim3 row_grid(long long rows, int row_len) {
-  return dim3((unsigned)cdiv(row_len, 256), (unsigned)(rows < 65535 ? rows : 65535));
-}
-
-static bool aligned16(const void* p) { return ((uintptr_t)p & 15u) == 0; }
 
 }  // namespace dgod
 

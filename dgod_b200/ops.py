@@ -1114,7 +1114,7 @@ def detect_candidates(class_logits: Tensor, box_regression: Tensor, proposals: T
 def _map_layout(t: Tensor) -> Tuple[Tensor, bool]:
     """(t as NHWC or NCHW dense fp32 memory, is NHWC).  A map whose two layouts coincide (1x1 pixels) runs as NCHW."""
     if t.dtype != torch.float32 or t.dim() != 4:
-        raise RuntimeError(f"FPN / stem kernels take float32 [N, C, H, W] maps, got {t.dtype} {tuple(t.shape)}")
+        raise RuntimeError(f"backbone kernels take float32 [N, C, H, W] maps, got {t.dtype} {tuple(t.shape)}")
     if t.is_contiguous():
         return t, False
     if t.is_contiguous(memory_format=torch.channels_last):
@@ -1227,3 +1227,57 @@ def stem_pool(conv: Tensor, shift: Tensor) -> Tensor:
     check(_lib.load().dgod_stem_pool_fwd(_p(conv), _p(shift), _p(out), n, h, w, c, ho, wo, int(nhwc), _stream()))
     KernelTimer.stop(tok)
     return out
+
+
+# --------------------------------------------------------------------------------- backbone: folded Bottleneck epilogue
+def _shift_relu_fwd(c: Tensor, shift: Tensor, residual: Optional[Tensor], res_shift: Optional[Tensor]) -> Tensor:
+    c, nhwc = _map_layout(c)
+    shift = _f32c(shift)
+    n, ch, h, w = c.shape
+    if residual is not None:
+        residual = _like(residual, nhwc)
+        if residual.dtype != torch.float32 or residual.shape != c.shape:
+            raise RuntimeError(f"shift_relu: residual {residual.dtype} {tuple(residual.shape)} does not match the "
+                               f"float32 {tuple(c.shape)} conv output")
+    if res_shift is not None:
+        res_shift = _f32c(res_shift)
+    if shift.shape != (ch,) or (res_shift is not None and res_shift.shape != (ch,)):
+        raise RuntimeError(f"shift_relu: shifts of shape ({ch},) expected, got {tuple(shift.shape)}"
+                           + ("" if res_shift is None else f" and {tuple(res_shift.shape)}"))
+    out = torch.empty_like(c)
+    tok = KernelTimer.start("shift_relu", 4 * c.numel() * (2 if residual is None else 3))
+    check(_lib.load().dgod_shift_relu_fwd(_p(c), _p(shift), _p(residual), _p(res_shift), _p(out), n, h, w, ch,
+                                          int(nhwc), _stream()))
+    KernelTimer.stop(tok)
+    return out
+
+
+class _ShiftReluFn(torch.autograd.Function):
+    """Forward: dgod_shift_relu_fwd.  Backward: the ReLU's threshold_backward — the kernel relu_'s autograd runs — and
+    that gradient for both `c` and the residual, as the adds' backward passes it on."""
+
+    @staticmethod
+    def forward(ctx, c, shift, residual, res_shift):
+        y = _shift_relu_fwd(c, shift, residual, res_shift)
+        ctx.save_for_backward(y)
+        return y
+
+    @staticmethod
+    def backward(ctx, g):
+        y, = ctx.saved_tensors
+        gc = torch.ops.aten.threshold_backward(g, y, 0)
+        return (gc if ctx.needs_input_grad[0] else None), None, (gc if ctx.needs_input_grad[2] else None), None
+
+
+def shift_relu(c: Tensor, shift: Tensor, residual: Optional[Tensor] = None, res_shift: Optional[Tensor] = None) -> Tensor:
+    """The epilogue of a folded ResNet Bottleneck convolution in one pass, bit-exact with torchvision's forward on the
+    folded convs (dgod_shift_relu_fwd):  relu(c + shift[c]) for conv1 / conv2; relu((c + shift) + residual) for the
+    tail of an identity block; relu((c + shift) + (residual + res_shift)) for the tail of a downsample block, whose
+    residual is the downsample conv's output without its shift.  `c` and `residual` may require grad; the shifts are
+    frozen-BN buffers and may not.  The result has c's memory layout."""
+    _need_cuda(c, shift, residual, res_shift)
+    if shift.requires_grad or (res_shift is not None and res_shift.requires_grad):
+        raise RuntimeError("shift_relu: the shifts are frozen (no gradient); got a shift that requires grad")
+    if res_shift is not None and residual is None:
+        raise ValueError("shift_relu: res_shift needs a residual")
+    return _ShiftReluFn.apply(c, shift, residual, res_shift)

@@ -3,6 +3,7 @@ from __future__ import annotations
 
 import torch
 from torch import nn
+from torchvision.models.resnet import Bottleneck
 
 
 @torch.no_grad()
@@ -55,6 +56,12 @@ class _FoldedConv2d(nn.Conv2d):
         scale, shift = self._scale_shift()
         return self._conv_forward(x, self.weight * scale.view(-1, 1, 1, 1), shift)
 
+    def _bias_free(self, x):
+        """(conv(x, w * s) without the shift, shift): the same cuDNN call as forward() makes, for a native epilogue
+        that adds the shift itself."""
+        scale, shift = self._scale_shift()
+        return self._conv_forward(x, self.weight * scale.view(-1, 1, 1, 1), None), shift
+
 
 class _FoldedStem(_FoldedConv2d):
     """The folded conv1 of a frozen ResNet stem together with the ReLU and 3x3 / stride-2 max-pool behind it.  On CUDA:
@@ -68,8 +75,7 @@ class _FoldedStem(_FoldedConv2d):
         if not x.is_cuda:
             return super().forward(x)
         from . import ops
-        scale, shift = self._scale_shift()
-        return ops.stem_pool(self._conv_forward(x, self.weight * scale.view(-1, 1, 1, 1), None), shift)
+        return ops.stem_pool(*self._bias_free(x))
 
 
 class _StemReLU(nn.ReLU):
@@ -84,6 +90,37 @@ class _StemMaxPool(nn.MaxPool2d):
 
     def forward(self, x):
         return x if x.is_cuda else super().forward(x)
+
+
+class _FusedBottleneck(Bottleneck):
+    """A torchvision Bottleneck whose convolutions (and downsample conv) are folded.  On CUDA: each cuDNN convolution
+    without its shift, then ONE native pass per convolution (ops.shift_relu) that adds the shift, the block's identity or
+    shifted downsample output, and applies the ReLU — where the stock forward makes a bias add, a ReLU and, at the
+    tail, a residual add (plus the downsample's bias add) as separate full-size passes.  The convolutions are the calls
+    ATen makes in the stock forward, so outputs and gradients are bit-identical.  On CPU it is the stock forward."""
+
+    def forward(self, x):
+        if not x.is_cuda:
+            return super().forward(x)
+        from . import ops
+        out = ops.shift_relu(*self.conv1._bias_free(x))
+        out = ops.shift_relu(*self.conv2._bias_free(out))
+        c, shift = self.conv3._bias_free(out)
+        if self.downsample is None:
+            return ops.shift_relu(c, shift, x)
+        return ops.shift_relu(c, shift, *self.downsample[0]._bias_free(x))
+
+
+def _fuse_bottleneck(block: nn.Module) -> None:
+    """Rebinds a torchvision Bottleneck whose conv1-3 (and downsample conv, if any) are folded to _FusedBottleneck."""
+    pairs = [(block.conv1, block.bn1), (block.conv2, block.bn2), (block.conv3, block.bn3)]
+    ds = block.downsample
+    if ds is not None:
+        if not (type(ds) is nn.Sequential and len(ds) == 2):
+            return
+        pairs.append((ds[0], ds[1]))
+    if type(block.relu) is nn.ReLU and all(type(c) is _FoldedConv2d and c._folded_bn[0] is bn for c, bn in pairs):
+        block.__class__ = _FusedBottleneck
 
 
 def _pair(v):
@@ -108,7 +145,8 @@ def _fuse_frozen_stem(parent: nn.Module) -> None:
 def fold_frozen_bn(module: nn.Module) -> int:
     """Rebinds every (Conv2d without bias, FrozenBatchNorm2d) sibling pair that torchvision's ResNet applies
     back to back (stem, Bottleneck conv1-3, downsample) so that the BN becomes the conv's epilogue.
-    A frozen stem additionally runs its shift, ReLU and max-pool as one native pass on CUDA (_FoldedStem).
+    A frozen stem additionally runs its shift, ReLU and max-pool as one native pass on CUDA (_FoldedStem), and every
+    folded Bottleneck its shifts, residual add and ReLUs as one native pass per convolution (_FusedBottleneck).
     Call after `calibrate_frozen_bn`.  State-dict keys and parameters are unchanged.  Returns the
     number of folded pairs; `unfold_frozen_bn` restores the stock modules."""
     from torchvision.ops.misc import FrozenBatchNorm2d
@@ -129,13 +167,18 @@ def fold_frozen_bn(module: nn.Module) -> int:
                 n += 1
             prev = child
         _fuse_frozen_stem(parent)
+    for m in module.modules():                     # after the loop above: a block's downsample is folded after the block
+        if type(m) is Bottleneck:
+            _fuse_bottleneck(m)
     return n
 
 
 def unfold_frozen_bn(module: nn.Module) -> None:
     from torchvision.ops.misc import FrozenBatchNorm2d
     for m in module.modules():
-        if type(m) is _StemReLU:
+        if type(m) is _FusedBottleneck:
+            m.__class__ = Bottleneck
+        elif type(m) is _StemReLU:
             m.__class__ = nn.ReLU
         elif type(m) is _StemMaxPool:
             m.__class__ = nn.MaxPool2d

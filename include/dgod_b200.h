@@ -35,6 +35,7 @@
  *   dgod_fpn_merge_fwd/_bwd TV ops/feature_pyramid_network.py FeaturePyramidNetwork.forward (lateral bias add, nearest
  *                           upsample, add) and its autograd (upsample_nearest2d_backward + accumulation)
  *   dgod_stem_pool_fwd      TV models/resnet.py ResNet._forward_impl: bn1 shift (folded), relu, maxpool of a frozen stem
+ *   dgod_shift_relu_fwd     TV models/resnet.py Bottleneck.forward: bn1-3 and downsample shifts (folded), residual add, relu
  */
 #ifndef DGOD_B200_H_
 #define DGOD_B200_H_
@@ -48,7 +49,7 @@ extern "C" {
 
 typedef void* dgod_stream_t; /* a cudaStream_t (0 = legacy default stream) */
 
-#define DGOD_ABI_VERSION 4
+#define DGOD_ABI_VERSION 5
 
 enum {
   DGOD_OK = 0,
@@ -349,10 +350,10 @@ int dgod_image_batch_u8(const uint8_t* const* images, const int* in_h, const int
 int dgod_nchw_to_nhwc(const void* src, void* dst, int batch, int channels, int hw, int dtype,
                       dgod_stream_t stream);
 
-/* ------------------------------------------------------------------ backbone boundary: FPN top-down merge, stem */
+/* ------------------------------------------------------------------ backbone: bottleneck epilogue, FPN top-down merge, stem */
 
 /* Maps are fp32 [n, c, h, w] in NCHW (channels_last = 0) or NHWC memory (channels_last = 1: c % 4 == 0 and every
- * pointer 16-byte aligned).  All three are bit-exact with the ATen ops they replace.
+ * pointer 16-byte aligned).  All of them are bit-exact with the ATen ops they replace.
  *
  * FPN merge: out = (lat + bias[c]) + nearest_upsample(coarse [n, c, hc, wc]) to [h, w], the two adds in that order, the
  * source pixel as ATen's nearest mode computes it (min(floor(y * ((float)hc / h)), hc - 1), likewise x).  out may be
@@ -369,6 +370,15 @@ int dgod_fpn_merge_bwd(const float* g_fine, const float* g_lb, float* g_coarse, 
  * ho = (h - 1) / 2 + 1, wo = (w - 1) / 2 + 1; NaN propagates as through clamp_min and max_pool2d.  No backward. */
 int dgod_stem_pool_fwd(const float* conv, const float* shift /*device [c]*/, float* out, int n, int h, int w, int c,
                        int ho, int wo, int channels_last, dgod_stream_t stream);
+
+/* Folded ResNet Bottleneck epilogue, one pass per convolution: out [n, c, h, w] = relu(conv + shift[c]) (conv1, conv2),
+ * relu((conv + shift[c]) + res) (identity block tail) or relu((conv + shift[c]) + (res + res_shift[c])) (downsample
+ * block tail: res is the downsample conv's output without its shift).  res and res_shift may be NULL (res_shift only
+ * with res).  Same layout rules as above for every map; bit-exact with ATen's adds in that order and relu_
+ * (clamp_min: NaN passes).  No backward: the gradient is threshold_backward(grad_out, out, 0) for conv and res. */
+int dgod_shift_relu_fwd(const float* conv, const float* shift /*device [c]*/, const float* res,
+                        const float* res_shift /*device [c]*/, float* out, int n, int h, int w, int c, int channels_last,
+                        dgod_stream_t stream);
 
 /* ------------------------------------------------------------------ gradient reversal */
 
