@@ -19,6 +19,7 @@ from torch import Tensor, nn
 
 from . import ops
 from .detector import FasterRCNN
+from .metrics import DetectionValidation
 
 
 class ImageDAFPN(nn.Module):
@@ -78,9 +79,10 @@ class InsCls(_InstanceMLP):
         super().__init__(num_cls, reverse=False)
 
 
-class DGFRCNN(nn.Module):
+class DGFRCNN(DetectionValidation, nn.Module):
     """DGFRCNN.py:73-201.  `training_step(batch)` returns the loss and advances the mode schedule;
-    `batch` = (images list, boxes list, labels list, domain tensor) like DGcommon.collate_fn."""
+    `batch` = (images list, boxes list, labels list, domain tensor) like DGcommon.collate_fn.  `validation_step` /
+    `on_validation_epoch_end` score the detector with mAP@0.5 (metrics.DetectionValidation)."""
 
     def __init__(self, n_classes: int, batch_size: int, exp: str, reg_weights: Sequence[float], num_domains: int,
                  min_size: int = 600, max_size: int = 1200, batched_modes: bool = True,

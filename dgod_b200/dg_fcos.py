@@ -31,6 +31,7 @@ from torchvision.ops.feature_pyramid_network import LastLevelP6P7
 
 from . import ops
 from .detector import FusedTransform
+from .metrics import DetectionValidation
 
 
 # --------------------------------------------------------------------------------- detector
@@ -201,10 +202,11 @@ class InsCls(_InsCls):
 
 
 # --------------------------------------------------------------------------------- DGFCOS
-class DGFCOS(nn.Module):
+class DGFCOS(DetectionValidation, nn.Module):
     """DGFCOS.py:115-243 without the Lightning trainer: `training_step(batch)` returns the loss of
     the current mode and advances the 0,1,0,2,0,3,0,4 schedule.  batch = (images, boxes, labels,
-    domain) as the reference's collate_fn yields them (DGcommon.py:14-31), tensors on the device."""
+    domain) as the reference's collate_fn yields them (DGcommon.py:14-31), tensors on the device.
+    `validation_step` / `on_validation_epoch_end` score the detector with mAP@0.5 (metrics.DetectionValidation)."""
 
     def __init__(self, n_classes: int, batch_size: int, exp: str, reg_weights: Sequence[float], num_domains: int,
                  min_size: int = 600, max_size: int = 1200):

@@ -6,6 +6,7 @@
 (fasterrcnn.py:412-416), the two Matchers (TV rpn.py:169, roi_heads.py:538), RPN box similarity
 (TV rpn.py:167), `filter_proposals` / target assignment (fused, sync-free variants) and, for
 FCOS, the location->target assignment inside `compute_loss` (fcos.py:503-550).
+`patch()` also binds the GPU `MeanAveragePrecision` in the reference's DG namespaces.
 `unpatch()` restores every binding.  After patching the ops require CUDA tensors.
 """
 from __future__ import annotations
@@ -16,7 +17,7 @@ from typing import Dict, List, Tuple
 
 import torch
 
-from . import ops
+from . import metrics, ops
 from .poolers import MultiScaleRoIAlign
 
 _saved: List[Tuple[object, str, object]] = []
@@ -44,12 +45,16 @@ def patch(grad_reverse: bool = True) -> None:
     _set(torchvision.ops, "roi_align", ops.roi_align)
     _set(torchvision.ops, "MultiScaleRoIAlign", MultiScaleRoIAlign)
     _set(det_utils, "Matcher", ops.Matcher)
-    if grad_reverse:
-        # DGFRCNN.py:1 / DGFCOS.py:1 do `from DGcommon import *`: rebind in every namespace
-        for name in ("DGcommon", "DGFRCNN", "DGFCOS"):
-            mod = sys.modules.get(name)
-            if mod is not None and hasattr(mod, "grad_reverse"):
-                _set(mod, "grad_reverse", ops.grad_reverse)
+    # DGFRCNN.py:1 / DGFCOS.py:1 do `from DGcommon import *`: rebind in every namespace.  The metric is looked up when
+    # a DGModel is constructed (DGcommon.py:127), so models built after patch() validate on the GPU metric.
+    for name in ("DGcommon", "DGFRCNN", "DGFCOS"):
+        mod = sys.modules.get(name)
+        if mod is None:
+            continue
+        if grad_reverse and hasattr(mod, "grad_reverse"):
+            _set(mod, "grad_reverse", ops.grad_reverse)
+        if hasattr(mod, "MeanAveragePrecision"):
+            _set(mod, "MeanAveragePrecision", metrics.MeanAveragePrecision)
 
 
 def unpatch() -> None:

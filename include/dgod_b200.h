@@ -36,6 +36,9 @@
  *                           upsample, add) and its autograd (upsample_nearest2d_backward + accumulation)
  *   dgod_stem_pool_fwd      TV models/resnet.py ResNet._forward_impl: bn1 shift (folded), relu, maxpool of a frozen stem
  *   dgod_shift_relu_fwd     TV models/resnet.py Bottleneck.forward: bn1-3 and downsample shifts (folded), residual add, relu
+ *   dgod_map_match          torchmetrics MeanAveragePrecision (pycocotools backend): COCOeval.computeIoU / evaluateImg,
+ *                           maskApi.c bbIou (DGcommon.py:127,154-172: the validation metric)
+ *   dgod_map_accumulate     the same: COCOeval.accumulate
  */
 #ifndef DGOD_B200_H_
 #define DGOD_B200_H_
@@ -49,7 +52,7 @@ extern "C" {
 
 typedef void* dgod_stream_t; /* a cudaStream_t (0 = legacy default stream) */
 
-#define DGOD_ABI_VERSION 5
+#define DGOD_ABI_VERSION 6
 
 enum {
   DGOD_OK = 0,
@@ -379,6 +382,36 @@ int dgod_stem_pool_fwd(const float* conv, const float* shift /*device [c]*/, flo
 int dgod_shift_relu_fwd(const float* conv, const float* shift /*device [c]*/, const float* res,
                         const float* res_shift /*device [c]*/, float* out, int n, int h, int w, int c, int channels_last,
                         dgod_stream_t stream);
+
+/* ------------------------------------------------------------------ validation mAP (COCO bbox, no crowd, area "all") */
+
+#define DGOD_MAP_MAX_DETS_PER_IMAGE 4096
+#define DGOD_MAP_MAX_GTS_PER_IMAGE 1024
+#define DGOD_MAP_MAX_IOU_THRESHOLDS 32
+
+/* Greedy matching of n_img images, one CTA each.  Detections (det_boxes [n,4] xyxy fp32, 16-byte aligned; det_scores
+ * [n] fp32; det_labels [n] int64) and ground truths (gt_boxes [m,4], gt_labels [m]) are concatenated over the images,
+ * image i owning rows [off[i], off[i+1]) of det_offsets / gt_offsets (device int32 [n_img+1]).  max_dets_per_image /
+ * max_gts_per_image bound every image's counts (they size shared memory; <= the caps above).  iou_thresholds: device
+ * double [n_thr], 1 <= n_thr <= 32.
+ * Per (image, label): detections in descending score order (stable; -0.0 ties +0.0), the first max_det kept; for each
+ * threshold t (as min(t, 1 - 1e-10)) each kept detection in turn takes the unmatched GT of its label with the largest
+ * IoU >= t, the later GT on equal IoU; IoU = pycocotools bbIou in double on the boxes converted to xywh in fp32.
+ * Writes, at every detection's own row: tp_mask (bit t set = matched at threshold t) and kept (1 = within max_det). */
+int dgod_map_match(const float* det_boxes, const float* det_scores, const int64_t* det_labels, const int* det_offsets,
+                   const float* gt_boxes, const int64_t* gt_labels, const int* gt_offsets, int n_img,
+                   int max_dets_per_image, int max_gts_per_image, const double* iou_thresholds, int n_thr, int max_det,
+                   uint32_t* tp_mask, uint8_t* kept, dgod_stream_t stream);
+/* Per-class precision / recall tables (COCOeval.accumulate), one CTA per (class, threshold).  tp_mask [n_records]: the
+ * kept detections' masks grouped by class and, within a class, in descending score order (ties: earlier image, then
+ * the image's own order); class k owns rows [seg_offsets[k], seg_offsets[k+1]) (device int32 [n_classes+1]; rows
+ * past the last segment are ignored); gt_counts: device int32 [n_classes]; rec_thresholds: device double [n_rec_thr].
+ * Writes precision [n_thr, n_rec_thr, n_classes] and recall [n_thr, n_classes] (float64; -1 for a class without
+ * ground truth).  Workspace: dgod_map_accumulate_workspace_bytes(n_records, n_thr). */
+size_t dgod_map_accumulate_workspace_bytes(int n_records, int n_thr);
+int dgod_map_accumulate(const uint32_t* tp_mask, const int* seg_offsets, const int* gt_counts, int n_classes,
+                        int n_records, const double* rec_thresholds, int n_rec_thr, int n_thr, double* precision,
+                        double* recall, void* workspace, size_t workspace_bytes, dgod_stream_t stream);
 
 /* ------------------------------------------------------------------ gradient reversal */
 
