@@ -106,6 +106,58 @@ __device__ __forceinline__ float float_from_ordered(uint32_t k) {
 // is ::max(v, 0), i.e. fmaxf — the same instruction, so signed zeros come out as ATen's do.
 __device__ __forceinline__ float clamp_min0(float v) { return isnan(v) ? v : fmaxf(v, 0.f); }
 
+// ---------------------------------------------------------------- storage types of the backbone epilogue kernels
+// Maps are stored as T (float or __nv_bfloat16) and computed on in fp32 ("opmath", as ATen does for bf16).  A 16-byte
+// access holds Pack<T>::N = 1 << Pack<T>::SHIFT values.  round_to<T> is the rounding an ATen op applies when its result
+// is a T tensor: none for float, round-to-nearest-even for bf16 (c10::BFloat16(float) is __float2bfloat16 on sm_80+).
+template <typename T> struct Pack;
+template <> struct Pack<float> {
+  static constexpr int N = 4, SHIFT = 2;
+  typedef float4 V;
+  __device__ __forceinline__ static void unpack(const float4 v, float (&f)[4]) {
+    f[0] = v.x; f[1] = v.y; f[2] = v.z; f[3] = v.w;
+  }
+  __device__ __forceinline__ static float4 pack(const float (&f)[4]) { return make_float4(f[0], f[1], f[2], f[3]); }
+};
+template <> struct Pack<__nv_bfloat16> {
+  static constexpr int N = 8, SHIFT = 3;
+  typedef uint4 V;
+  __device__ __forceinline__ static void unpack(const uint4 v, float (&f)[8]) {
+    const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      f[2 * i] = __uint_as_float(w[i] << 16);
+      f[2 * i + 1] = __uint_as_float(w[i] & 0xffff0000u);
+    }
+  }
+  __device__ __forceinline__ static uint4 pack(const float (&f)[8]) {
+    uint32_t w[4];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      const __nv_bfloat162 h = __floats2bfloat162_rn(f[2 * i], f[2 * i + 1]);
+      w[i] = *reinterpret_cast<const uint32_t*>(&h);
+    }
+    return make_uint4(w[0], w[1], w[2], w[3]);
+  }
+};
+
+__device__ __forceinline__ float to_f(float v) { return v; }
+__device__ __forceinline__ float to_f(__nv_bfloat16 v) { return __bfloat162float(v); }
+template <typename T> __device__ __forceinline__ T from_f(float v);
+template <> __device__ __forceinline__ float from_f<float>(float v) { return v; }
+template <> __device__ __forceinline__ __nv_bfloat16 from_f<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
+template <typename T> __device__ __forceinline__ float round_to(float v) { return to_f(from_f<T>(v)); }
+
+// The N fp32 per-channel values (shifts, biases) that go with 16-byte map vector `i`: p must be 16-byte aligned.
+template <int N>
+__device__ __forceinline__ void ldg_channels(const float* __restrict__ p, int i, float (&f)[N]) {
+#pragma unroll
+  for (int k = 0; k < N / 4; ++k) {
+    const float4 v = __ldg(reinterpret_cast<const float4*>(p) + i * (N / 4) + k);
+    f[4 * k] = v.x; f[4 * k + 1] = v.y; f[4 * k + 2] = v.z; f[4 * k + 3] = v.w;
+  }
+}
+
 // Streaming passes over [rows x row_len] maps: rows go to the grid's y dimension (at most 65535, the kernels stride over
 // the rest), a row's elements to x in blocks of 256 threads.
 static inline dim3 row_grid(long long rows, int row_len) {

@@ -351,8 +351,18 @@ class FusedFPN(FeaturePyramidNetwork):
             return super().forward(x)
         convs = [blk[0] for blk in self.inner_blocks]
         top = self.inner_blocks[-1](feats[-1])
-        laterals = [conv._conv_forward(f, conv.weight, None) for conv, f in zip(convs[:-1], feats[:-1])]
-        inners = ops.fpn_top_down(laterals, [conv.bias for conv in convs[:-1]], top)
+        if torch.is_autocast_enabled("cuda"):
+            # Under autocast F.interpolate runs in fp32 (upsample_nearest2d is on autocast's fp32 list), so the stock
+            # merge adds a bf16 lateral, bias included, to an fp32 map: every merged level but the top is fp32.  The fp32
+            # merge on the upcast laterals computes exactly that; their bias is already in, so it adds -0.0 (an exact
+            # identity).  The top feeds its layer block as the bf16 map the stock forward uses.
+            laterals = [conv(f).float() for conv, f in zip(convs[:-1], feats[:-1])]
+            no_bias = [torch.full((conv.out_channels,), -0.0, device=top.device) for conv in convs[:-1]]
+            inners = ops.fpn_top_down(laterals, no_bias, top.float())
+            inners[-1] = top
+        else:
+            laterals = [conv._conv_forward(f, conv.weight, None) for conv, f in zip(convs[:-1], feats[:-1])]
+            inners = ops.fpn_top_down(laterals, [conv.bias for conv in convs[:-1]], top)
         results = [blk(t) for blk, t in zip(self.layer_blocks, inners)]
         if self.extra_blocks is not None:
             results, names = self.extra_blocks(results, feats, names)

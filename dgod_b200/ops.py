@@ -571,8 +571,10 @@ def fcos_loss(cls_logits: Tensor, bbox_regression: Tensor, bbox_ctrness: Tensor,
     outputs, no host sync.  cls_logits [B,N,C], bbox_regression [B,N,4], bbox_ctrness [B,N,1] fp32;
     anchors [N,4]; cls_targets [B,N] int64 (-1 = background) and box_targets [B,N,4] from `fcos_assign`."""
     for t in (cls_logits, bbox_regression, bbox_ctrness):
-        if t.dtype != torch.float32:
-            raise RuntimeError(f"fcos_loss: float32 head outputs expected, got {t.dtype}")
+        if t.dtype not in (torch.float32, torch.bfloat16):
+            raise RuntimeError(f"fcos_loss: float32 or bfloat16 head outputs expected, got {t.dtype}")
+    # bf16 head outputs (autocast) go through the fp32 loss kernels, as autocast runs the stock losses in fp32
+    cls_logits, bbox_regression, bbox_ctrness = cls_logits.float(), bbox_regression.float(), bbox_ctrness.float()
     B, N, _ = cls_logits.shape
     if bbox_regression.shape != (B, N, 4) or bbox_ctrness.numel() != B * N or cls_targets.shape != (B, N):
         raise RuntimeError("fcos_loss: expected cls_logits [B,N,C], bbox_regression [B,N,4], bbox_ctrness [B,N,1], "
@@ -881,6 +883,8 @@ class _GRLLinear(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gy):
         x, w = ctx.saved_tensors
+        # Under autocast the forward ran in gy's dtype: the GEMMs take the operands autocast gave F.linear.
+        x, w = x.to(gy.dtype), w.to(gy.dtype)
         gx = gw = gb = None
         gy2 = gy.reshape(-1, gy.shape[-1])
         if ctx.needs_input_grad[0]:
@@ -913,6 +917,7 @@ class _GRLConv2d(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gy):
         x, w = ctx.saved_tensors
+        x, w = x.to(gy.dtype), w.to(gy.dtype)         # under autocast: the operands autocast gave F.conv2d
         stride, padding, dilation, groups, alpha, bias_sizes = ctx.cfg
         gx = gw = gb = None
         common = (list(stride), list(padding), list(dilation), False, [0, 0], groups)
@@ -1112,9 +1117,10 @@ def detect_candidates(class_logits: Tensor, box_regression: Tensor, proposals: T
 
 # --------------------------------------------------------------------------------- backbone boundary: FPN merge, stem
 def _map_layout(t: Tensor) -> Tuple[Tensor, bool]:
-    """(t as NHWC or NCHW dense fp32 memory, is NHWC).  A map whose two layouts coincide (1x1 pixels) runs as NCHW."""
-    if t.dtype != torch.float32 or t.dim() != 4:
-        raise RuntimeError(f"backbone kernels take float32 [N, C, H, W] maps, got {t.dtype} {tuple(t.shape)}")
+    """(t as NHWC or NCHW dense memory, is NHWC).  A map whose two layouts coincide (1x1 pixels) runs as NCHW."""
+    if t.dtype not in (torch.float32, torch.bfloat16) or t.dim() != 4:
+        raise RuntimeError(f"backbone kernels take [N, C, H, W] maps (float32 and bfloat16 only), got {t.dtype} "
+                           f"{tuple(t.shape)}")
     if t.is_contiguous():
         return t, False
     if t.is_contiguous(memory_format=torch.channels_last):
@@ -1126,20 +1132,27 @@ def _like(t: Tensor, nhwc: bool) -> Tensor:
     return t.contiguous(memory_format=torch.channels_last if nhwc else torch.contiguous_format)
 
 
+def _map_fn(name: str, t: Tensor):
+    """The C entry point `name` for maps of t's dtype: the fp32 one or its `_bf16` sibling."""
+    lib = _lib.load()
+    return getattr(lib, name) if t.dtype == torch.float32 else getattr(lib, name + "_bf16")
+
+
 def fpn_merge(lat: Tensor, bias: Tensor, coarse: Tensor) -> Tensor:
     """(lat + bias[c]) + F.interpolate(coarse, size=lat.shape[-2:], mode="nearest") in one pass, bit-exact
-    (dgod_fpn_merge_fwd); the result has lat's memory layout."""
+    (dgod_fpn_merge_fwd, or dgod_fpn_merge_fwd_bf16 for bf16 maps: then as under autocast, the fp32 bias rounded to bf16
+    first); the result has lat's memory layout and dtype."""
     _need_cuda(lat, bias, coarse)
     lat, nhwc = _map_layout(lat)
     coarse, bias = _like(coarse, nhwc), _f32c(bias)
     n, c, h, w = lat.shape
-    if coarse.dtype != torch.float32 or coarse.shape[:2] != lat.shape[:2] or bias.shape != (c,):
-        raise RuntimeError(f"fpn_merge: lateral {tuple(lat.shape)}, bias {tuple(bias.shape)} and coarse "
-                           f"{tuple(coarse.shape)} float32 maps of one batch and channel count expected")
+    if coarse.dtype != lat.dtype or coarse.shape[:2] != lat.shape[:2] or bias.shape != (c,):
+        raise RuntimeError(f"fpn_merge: lateral {lat.dtype} {tuple(lat.shape)}, bias {tuple(bias.shape)} and coarse "
+                           f"{coarse.dtype} {tuple(coarse.shape)}: maps of one dtype, batch and channel count expected")
     out = torch.empty_like(lat)
-    tok = KernelTimer.start("fpn_merge_fwd", 4 * (2 * lat.numel() + coarse.numel()))
-    check(_lib.load().dgod_fpn_merge_fwd(_p(lat), _p(bias), _p(coarse), _p(out), n, h, w, coarse.shape[2],
-                                         coarse.shape[3], c, int(nhwc), _stream()))
+    tok = KernelTimer.start("fpn_merge_fwd", lat.element_size() * (2 * lat.numel() + coarse.numel()))
+    check(_map_fn("dgod_fpn_merge_fwd", lat)(_p(lat), _p(bias), _p(coarse), _p(out), n, h, w, coarse.shape[2],
+                                             coarse.shape[3], c, int(nhwc), _stream()))
     KernelTimer.stop(tok)
     return out
 
@@ -1154,15 +1167,18 @@ def fpn_merge_backward(g_fine: Optional[Tensor], g_lb: Optional[Tensor], coarse_
     n, c, h, w = g_fine.shape
     if g_lb is not None:
         g_lb = _like(g_lb, nhwc)
-        if g_lb.dtype != torch.float32 or tuple(g_lb.shape) != tuple(coarse_shape):
-            raise RuntimeError(f"fpn_merge_backward: gradient {tuple(g_lb.shape)} of the {tuple(coarse_shape)} level")
+        if g_lb.dtype != g_fine.dtype or tuple(g_lb.shape) != tuple(coarse_shape):
+            raise RuntimeError(f"fpn_merge_backward: gradient {g_lb.dtype} {tuple(g_lb.shape)} of the "
+                               f"{tuple(coarse_shape)} level, {g_fine.dtype} expected")
         out = torch.empty_like(g_lb)
     else:
-        out = torch.empty(tuple(coarse_shape), dtype=torch.float32, device=g_fine.device,
+        out = torch.empty(tuple(coarse_shape), dtype=g_fine.dtype, device=g_fine.device,
                           memory_format=torch.channels_last if nhwc else torch.contiguous_format)
     hc, wc = out.shape[2], out.shape[3]
-    tok = KernelTimer.start("fpn_merge_bwd", 4 * (g_fine.numel() + (2 if g_lb is not None else 1) * out.numel()))
-    check(_lib.load().dgod_fpn_merge_bwd(_p(g_fine), _p(g_lb), _p(out), n, h, w, hc, wc, c, int(nhwc), _stream()))
+    tok = KernelTimer.start("fpn_merge_bwd", g_fine.element_size() * (g_fine.numel() + (2 if g_lb is not None else 1)
+                                                                        * out.numel()))
+    check(_map_fn("dgod_fpn_merge_bwd", g_fine)(_p(g_fine), _p(g_lb), _p(out), n, h, w, hc, wc, c, int(nhwc),
+                                                _stream()))
     KernelTimer.stop(tok)
     return out
 
@@ -1221,10 +1237,10 @@ def stem_pool(conv: Tensor, shift: Tensor) -> Tensor:
     if shift.shape != (c,):
         raise RuntimeError(f"stem_pool: shift of shape ({c},) expected, got {tuple(shift.shape)}")
     ho, wo = (h - 1) // 2 + 1, (w - 1) // 2 + 1
-    out = torch.empty((n, c, ho, wo), dtype=torch.float32, device=conv.device,
+    out = torch.empty((n, c, ho, wo), dtype=conv.dtype, device=conv.device,
                       memory_format=torch.channels_last if nhwc else torch.contiguous_format)
-    tok = KernelTimer.start("stem_pool", 4 * (conv.numel() + out.numel()))
-    check(_lib.load().dgod_stem_pool_fwd(_p(conv), _p(shift), _p(out), n, h, w, c, ho, wo, int(nhwc), _stream()))
+    tok = KernelTimer.start("stem_pool", conv.element_size() * (conv.numel() + out.numel()))
+    check(_map_fn("dgod_stem_pool_fwd", conv)(_p(conv), _p(shift), _p(out), n, h, w, c, ho, wo, int(nhwc), _stream()))
     KernelTimer.stop(tok)
     return out
 
@@ -1236,18 +1252,18 @@ def _shift_relu_fwd(c: Tensor, shift: Tensor, residual: Optional[Tensor], res_sh
     n, ch, h, w = c.shape
     if residual is not None:
         residual = _like(residual, nhwc)
-        if residual.dtype != torch.float32 or residual.shape != c.shape:
+        if residual.dtype != c.dtype or residual.shape != c.shape:
             raise RuntimeError(f"shift_relu: residual {residual.dtype} {tuple(residual.shape)} does not match the "
-                               f"float32 {tuple(c.shape)} conv output")
+                               f"{c.dtype} {tuple(c.shape)} conv output")
     if res_shift is not None:
         res_shift = _f32c(res_shift)
     if shift.shape != (ch,) or (res_shift is not None and res_shift.shape != (ch,)):
         raise RuntimeError(f"shift_relu: shifts of shape ({ch},) expected, got {tuple(shift.shape)}"
                            + ("" if res_shift is None else f" and {tuple(res_shift.shape)}"))
     out = torch.empty_like(c)
-    tok = KernelTimer.start("shift_relu", 4 * c.numel() * (2 if residual is None else 3))
-    check(_lib.load().dgod_shift_relu_fwd(_p(c), _p(shift), _p(residual), _p(res_shift), _p(out), n, h, w, ch,
-                                          int(nhwc), _stream()))
+    tok = KernelTimer.start("shift_relu", c.element_size() * c.numel() * (2 if residual is None else 3))
+    check(_map_fn("dgod_shift_relu_fwd", c)(_p(c), _p(shift), _p(residual), _p(res_shift), _p(out), n, h, w, ch,
+                                            int(nhwc), _stream()))
     KernelTimer.stop(tok)
     return out
 

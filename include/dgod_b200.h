@@ -36,6 +36,8 @@
  *                           upsample, add) and its autograd (upsample_nearest2d_backward + accumulation)
  *   dgod_stem_pool_fwd      TV models/resnet.py ResNet._forward_impl: bn1 shift (folded), relu, maxpool of a frozen stem
  *   dgod_shift_relu_fwd     TV models/resnet.py Bottleneck.forward: bn1-3 and downsample shifts (folded), residual add, relu
+ *   dgod_*_bf16             the four backbone entry points above on bf16 maps: the same modules under
+ *                           torch.autocast("cuda", dtype=torch.bfloat16)
  *   dgod_map_match          torchmetrics MeanAveragePrecision (pycocotools backend): COCOeval.computeIoU / evaluateImg,
  *                           maskApi.c bbIou (DGcommon.py:127,154-172: the validation metric)
  *   dgod_map_accumulate     the same: COCOeval.accumulate
@@ -52,7 +54,7 @@ extern "C" {
 
 typedef void* dgod_stream_t; /* a cudaStream_t (0 = legacy default stream) */
 
-#define DGOD_ABI_VERSION 6
+#define DGOD_ABI_VERSION 7
 
 enum {
   DGOD_OK = 0,
@@ -382,6 +384,20 @@ int dgod_stem_pool_fwd(const float* conv, const float* shift /*device [c]*/, flo
 int dgod_shift_relu_fwd(const float* conv, const float* shift /*device [c]*/, const float* res,
                         const float* res_shift /*device [c]*/, float* out, int n, int h, int w, int c, int channels_last,
                         dgod_stream_t stream);
+
+/* The same four on bf16 maps (__nv_bfloat16 [n, c, h, w]; channels_last needs c % 8 == 0 and 16-byte aligned pointers);
+ * biases and shifts stay fp32.  Bit-exact with the ATen bf16 ops under autocast: fp32 math, every add's result rounded
+ * to bf16 (round to nearest even), each bias / shift rounded to bf16 before it is added (autocast casts a conv's bias),
+ * and the merge backward's window sum rounded once to bf16 before g_lb is added. */
+int dgod_fpn_merge_fwd_bf16(const void* lat, const float* bias /*device [c]*/, const void* coarse, void* out, int n,
+                            int h, int w, int hc, int wc, int c, int channels_last, dgod_stream_t stream);
+int dgod_fpn_merge_bwd_bf16(const void* g_fine, const void* g_lb, void* g_coarse, int n, int h, int w, int hc, int wc,
+                            int c, int channels_last, dgod_stream_t stream);
+int dgod_stem_pool_fwd_bf16(const void* conv, const float* shift /*device [c]*/, void* out, int n, int h, int w, int c,
+                            int ho, int wo, int channels_last, dgod_stream_t stream);
+int dgod_shift_relu_fwd_bf16(const void* conv, const float* shift /*device [c]*/, const void* res,
+                             const float* res_shift /*device [c]*/, void* out, int n, int h, int w, int c,
+                             int channels_last, dgod_stream_t stream);
 
 /* ------------------------------------------------------------------ validation mAP (COCO bbox, no crowd, area "all") */
 
