@@ -17,7 +17,7 @@ OBJ_DIR = PKG_DIR / "build"
 LIB_PATH = PKG_DIR / "libdgod_b200.so"
 SOURCES = ["error.cu", "tmap.cu", "match.cu", "fcos.cu", "fcos_loss.cu", "fcos_post.cu", "sampler.cu", "nms.cu", "rpn.cu", "roi_align.cu",
            "roi_align_fast.cu", "roi_align_tma.cu", "roi_align_own.cu", "misc.cu", "transform.cu",
-           "fpn.cu", "bottleneck.cu", "map_eval.cu"]
+           "fpn.cu", "bottleneck.cu", "map_eval.cu", "linear_tc.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
@@ -28,6 +28,9 @@ NVCC_FLAGS = [
     "-fmad=false",
     "-Xptxas", "-v",
 ]
+# DGOD_DEBUG_WAITS=1: bounded mbarrier waits in the tcgen05 kernels (a lost arrive is reported instead of hanging).
+if os.environ.get("DGOD_DEBUG_WAITS"):
+    NVCC_FLAGS.append("-DDGOD_DEBUG_WAITS")
 
 
 def _nvcc() -> str:

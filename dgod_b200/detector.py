@@ -126,6 +126,8 @@ class TwoMLPHead(nn.Module):
 
     def forward(self, x: Tensor, box_labels=None) -> Tensor:
         x = x.flatten(start_dim=1)
+        if ops.box_head_mlp_supported(x, self.fc6.weight, self.fc7.weight):
+            return ops.box_head_mlp(x, self.fc6.weight, self.fc6.bias, self.fc7.weight, self.fc7.bias)
         return F.relu(self.fc7(F.relu(self.fc6(x))))
 
 

@@ -902,6 +902,71 @@ def grl_linear(x: Tensor, weight: Tensor, bias: Optional[Tensor], alpha: float =
     return _GRLLinear.apply(x, weight, bias, alpha)
 
 
+# --------------------------------------------------------------------------------- box head MLP (fc6 / fc7)
+def linear_tc(a: Tensor, b: Tensor, *, a_trans: bool = False, b_trans: bool = False, bias: Optional[Tensor] = None,
+              relu: bool = False, mask: Optional[Tensor] = None, name: str = "linear_tc") -> Tensor:
+    """fp32 C = A @ B^T on the tensor cores, fp32-accurate (dgod_linear_tc, 3xTF32).  A is `a` [m, k] (or `a`^T when
+    a_trans: `a` is [k, m]), B is `b` [n, k] (or `b`^T: [k, n]).  Then + bias, ReLU, * (mask > 0), in that order."""
+    _need_cuda(a, b, bias, mask)
+    for t in (a, b, bias, mask):
+        if t is not None and (t.dtype != torch.float32 or not t.is_contiguous()):
+            raise ValueError("linear_tc: operands must be contiguous float32")
+    if a.dim() != 2 or b.dim() != 2:
+        raise ValueError("linear_tc: a and b must be 2-D")
+    m, k = (a.shape[1], a.shape[0]) if a_trans else a.shape
+    n, kb = (b.shape[1], b.shape[0]) if b_trans else b.shape
+    if k != kb:
+        raise ValueError(f"linear_tc: inner dimensions differ ({k} vs {kb})")
+    if bias is not None and bias.shape != (n,):
+        raise ValueError("linear_tc: bias must be [n]")
+    if mask is not None and mask.shape != (m, n):
+        raise ValueError("linear_tc: mask must be [m, n]")
+    lib = _lib.load()
+    c = torch.empty((m, n), dtype=torch.float32, device=a.device)
+    wsb = lib.dgod_linear_tc_workspace_bytes(m, n, k)
+    ws = _ws(wsb, a.device)
+    tok = KernelTimer.start(name, 4 * (m * k + n * k + m * n))
+    check(lib.dgod_linear_tc(_p(a), int(a_trans), _p(b), int(b_trans), m, n, k, _p(bias), int(relu), _p(mask), _p(c),
+                             _p(ws), ws.numel(), _stream()), ValueError)
+    KernelTimer.stop(tok)
+    return c
+
+
+def box_head_mlp_supported(x: Tensor, w6: Tensor, w7: Tensor) -> bool:
+    """Whether box_head_mlp takes these operands: CUDA fp32, autocast off, fc widths multiples of 32, x 16-byte aligned."""
+    return (x.is_cuda and x.dim() == 2 and x.dtype == torch.float32 and w6.dtype == torch.float32
+            and w7.dtype == torch.float32 and not torch.is_autocast_enabled("cuda") and x.shape[0] >= 1
+            and x.shape[1] >= 1 and x.data_ptr() % 16 == 0 and w6.shape[1] == x.shape[1] and w6.shape[0] % 32 == 0
+            and w7.shape == (w7.shape[0], w6.shape[0]) and w7.shape[0] % 32 == 0)
+
+
+class _BoxHeadMLP(torch.autograd.Function):
+    """relu(fc7(relu(fc6(x)))) on dgod_linear_tc: both ReLUs in the forward products' epilogues, fc6's ReLU mask in
+    the epilogue of fc7's input-gradient product.  fc7's ReLU backward and the bias gradients stay ATen."""
+
+    @staticmethod
+    def forward(ctx, x, w6, b6, w7, b7):
+        h6 = linear_tc(x, w6, bias=b6, relu=True, name="linear_tc_fwd")
+        h7 = linear_tc(h6, w7, bias=b7, relu=True, name="linear_tc_fwd")
+        ctx.save_for_backward(x, w6, w7, h6, h7)
+        return h7
+
+    @staticmethod
+    def backward(ctx, g7):
+        x, w6, w7, h6, h7 = ctx.saved_tensors
+        g7 = torch.ops.aten.threshold_backward(g7.contiguous(), h7, 0)
+        gw7 = linear_tc(g7, h6, a_trans=True, b_trans=True, name="linear_tc_wgrad")
+        g6 = linear_tc(g7, w7, b_trans=True, mask=h6, name="linear_tc_dgrad")
+        gw6 = linear_tc(g6, x, a_trans=True, b_trans=True, name="linear_tc_wgrad")
+        gx = linear_tc(g6, w6, b_trans=True, name="linear_tc_dgrad") if ctx.needs_input_grad[0] else None
+        return gx, gw6, g6.sum(0), gw7, g7.sum(0)
+
+
+def box_head_mlp(x: Tensor, w6: Tensor, b6: Tensor, w7: Tensor, b7: Tensor) -> Tensor:
+    """relu(linear(relu(linear(x, w6, b6)), w7, b7)) for fp32 x [m, k] with fp32 accuracy on the tensor cores."""
+    return _BoxHeadMLP.apply(x.contiguous(), w6.contiguous(), b6.contiguous(), w7.contiguous(), b7.contiguous())
+
+
 class _GRLConv2d(torch.autograd.Function):
     """grad_reverse followed by nn.Conv2d with the reversal scale folded into the convolution's input-gradient
     (DGcommon.py:73-74 ImageDAFPN.Conv1, DGcommon.py:106-107 ImageDA.Conv1): cuDNN's dgrad runs on the weight

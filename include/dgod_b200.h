@@ -41,6 +41,8 @@
  *   dgod_map_match          torchmetrics MeanAveragePrecision (pycocotools backend): COCOeval.computeIoU / evaluateImg,
  *                           maskApi.c bbIou (DGcommon.py:127,154-172: the validation metric)
  *   dgod_map_accumulate     the same: COCOeval.accumulate
+ *   dgod_linear_tc          TV models/detection/faster_rcnn.py TwoMLPHead (fasterrcnn.py:331-352): fc6 / fc7 Linear
+ *                           forward (bias, ReLU) and their autograd products, fp32-accurate on the tensor cores
  */
 #ifndef DGOD_B200_H_
 #define DGOD_B200_H_
@@ -54,7 +56,7 @@ extern "C" {
 
 typedef void* dgod_stream_t; /* a cudaStream_t (0 = legacy default stream) */
 
-#define DGOD_ABI_VERSION 7
+#define DGOD_ABI_VERSION 8
 
 enum {
   DGOD_OK = 0,
@@ -428,6 +430,19 @@ size_t dgod_map_accumulate_workspace_bytes(int n_records, int n_thr);
 int dgod_map_accumulate(const uint32_t* tp_mask, const int* seg_offsets, const int* gt_counts, int n_classes,
                         int n_records, const double* rec_thresholds, int n_rec_thr, int n_thr, double* precision,
                         double* recall, void* workspace, size_t workspace_bytes, dgod_stream_t stream);
+
+/* ------------------------------------------------------------------ fp32 matrix product (box head) */
+
+/* C [m, n] = epilogue(A B^T) on the tcgen05 tensor cores, fp32-accurate (3xTF32: each operand split into two tf32
+ * parts, three products accumulated in fp32; NaN / inf propagate to the same positions as in an fp32 SGEMM, where
+ * SGEMM gives +-inf this may give NaN).  A [m, k] is `a` stored [m, k] row-major, or with a_trans the transpose of
+ * `a` stored [k, m]; B [n, k] likewise from `b` ([n, k], or [k, n] with b_trans).  Epilogue, in this order: + bias[n]
+ * (device [n] or NULL), ReLU if relu (NaN passes), C *= (mask > 0) with mask device [m, n] or NULL.  c: device [m, n].
+ * m, k >= 1, n % 32 == 0, every pointer 16-byte aligned.  Workspace: dgod_linear_tc_workspace_bytes(m, n, k) (the
+ * split operands; 0 for invalid sizes). */
+size_t dgod_linear_tc_workspace_bytes(int m, int n, int k);
+int dgod_linear_tc(const float* a, int a_trans, const float* b, int b_trans, int m, int n, int k, const float* bias,
+                   int relu, const float* mask, float* c, void* workspace, size_t workspace_bytes, dgod_stream_t stream);
 
 /* ------------------------------------------------------------------ gradient reversal */
 
