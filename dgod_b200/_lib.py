@@ -15,7 +15,7 @@ LIB_PATH = PKG_DIR / "libdgod_b200.so"
 MAX_LEVELS = 8
 MAX_CELL_ANCHORS = 16
 F32, BF16 = 0, 1
-ABI_VERSION = 8   # DGOD_ABI_VERSION of include/dgod_b200.h
+ABI_VERSION = 9   # DGOD_ABI_VERSION of include/dgod_b200.h
 
 vp, i32, i64, f32, f64, sz = C.c_void_p, C.c_int, C.c_int64, C.c_float, C.c_double, C.c_size_t
 
@@ -88,6 +88,7 @@ SIGNATURES = {
     "dgod_fpn_merge_bwd": (i32, [vp, vp, vp, i32, i32, i32, i32, i32, i32, i32, vp]),
     "dgod_stem_pool_fwd": (i32, [vp, vp, vp, i32, i32, i32, i32, i32, i32, i32, vp]),
     "dgod_shift_relu_fwd": (i32, [vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, vp]),
+    "dgod_bias_add_fwd": (i32, [vp, vp, vp, i32, i32, i32, i32, i32, vp]),
     "dgod_fpn_merge_fwd_bf16": (i32, [vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, i32, vp]),
     "dgod_fpn_merge_bwd_bf16": (i32, [vp, vp, vp, i32, i32, i32, i32, i32, i32, i32, vp]),
     "dgod_stem_pool_fwd_bf16": (i32, [vp, vp, vp, i32, i32, i32, i32, i32, i32, i32, vp]),
@@ -97,6 +98,11 @@ SIGNATURES = {
     "dgod_map_accumulate": (i32, [vp, vp, vp, i32, i32, vp, i32, i32, vp, vp, vp, sz, vp]),
     "dgod_linear_tc_workspace_bytes": (sz, [i32, i32, i32]),
     "dgod_linear_tc": (i32, [vp, i32, vp, i32, i32, i32, i32, vp, i32, vp, vp, vp, sz, vp]),
+    "dgod_rpn_head_workspace_bytes": (sz, []),
+    "dgod_rpn_head_fwd": (i32, [C.POINTER(vp), i32, C.POINTER(i32), C.POINTER(i32), i32, i32, i32, vp, vp, vp, vp, vp,
+                                C.POINTER(vp), C.POINTER(vp), vp]),
+    "dgod_rpn_head_bwd": (i32, [C.POINTER(vp), i32, C.POINTER(i32), C.POINTER(i32), i32, i32, i32, vp, vp, vp,
+                                C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), vp, vp, sz, vp]),
 }
 
 _lib = None

@@ -17,7 +17,7 @@ OBJ_DIR = PKG_DIR / "build"
 LIB_PATH = PKG_DIR / "libdgod_b200.so"
 SOURCES = ["error.cu", "tmap.cu", "match.cu", "fcos.cu", "fcos_loss.cu", "fcos_post.cu", "sampler.cu", "nms.cu", "rpn.cu", "roi_align.cu",
            "roi_align_fast.cu", "roi_align_tma.cu", "roi_align_own.cu", "misc.cu", "transform.cu",
-           "fpn.cu", "bottleneck.cu", "map_eval.cu", "linear_tc.cu"]
+           "fpn.cu", "bottleneck.cu", "map_eval.cu", "linear_tc.cu", "rpn_head.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -11,6 +11,7 @@
 // bf16 maps (the block under torch.autocast(dtype=bfloat16)): fp32 math, and every add's result rounded to bf16 (RNE);
 // the fp32 shifts are rounded to bf16 first, as autocast casts the conv's bias before ATen's add_:
 //   v = bf16(c + bf16(s)), then bf16(v + r) (identity tail) or bf16(v + bf16(r + bf16(t))) (downsample tail), relu_.
+// dgod_bias_add_fwd is the fp32 SR_PLAIN instance without the ReLU: out = c + s (an FPN layer block's bias).
 // NHWC: one thread owns one 16-byte vector of a pixel's channels (4 fp32 or 8 bf16: C % 4 or C % 8 == 0), the grid's y
 // dimension walks the rows (n, y); NCHW: one element per thread, the grid's y dimension walks the planes (n, c).  Both
 // grid-stride.
@@ -21,15 +22,15 @@ namespace dgod {
 enum { SR_PLAIN = 0, SR_RESIDUAL = 1, SR_SHIFTED_RESIDUAL = 2 };
 
 // The shifts s and t arrive rounded to T (a bf16 conv's bias is cast to bf16 by autocast and added by a separate add_).
-template <typename T, int FORM>
+template <typename T, int FORM, bool RELU>
 __device__ __forceinline__ float shift_relu1(float c, float s, float r, float t) {
   float v = round_to<T>(__fadd_rn(c, s));
   if (FORM == SR_RESIDUAL) v = round_to<T>(__fadd_rn(v, r));
   if (FORM == SR_SHIFTED_RESIDUAL) v = round_to<T>(__fadd_rn(v, round_to<T>(__fadd_rn(r, t))));
-  return clamp_min0(v);
+  return RELU ? clamp_min0(v) : v;
 }
 
-template <typename T, bool NHWC, int FORM>
+template <typename T, bool NHWC, int FORM, bool RELU>
 __global__ void __launch_bounds__(256)
 shift_relu_kernel(const T* __restrict__ conv, const float* __restrict__ shift, const T* __restrict__ res,
                   const float* __restrict__ res_shift, T* __restrict__ out, int rows, int row_len, int C) {
@@ -49,7 +50,7 @@ shift_relu_kernel(const T* __restrict__ conv, const float* __restrict__ shift, c
         if (FORM != SR_PLAIN) Pack<T>::unpack(reinterpret_cast<const V*>(res)[row + j], q);
         if (FORM == SR_SHIFTED_RESIDUAL) ldg_channels<N>(res_shift, cv, t);
 #pragma unroll
-        for (int k = 0; k < N; ++k) v[k] = shift_relu1<T, FORM>(v[k], round_to<T>(s[k]), q[k], round_to<T>(t[k]));
+        for (int k = 0; k < N; ++k) v[k] = shift_relu1<T, FORM, RELU>(v[k], round_to<T>(s[k]), q[k], round_to<T>(t[k]));
         reinterpret_cast<V*>(out)[row + j] = Pack<T>::pack(v);
       }
     } else {
@@ -57,30 +58,34 @@ shift_relu_kernel(const T* __restrict__ conv, const float* __restrict__ shift, c
       const float s = round_to<T>(__ldg(shift + ch));
       const float t = FORM == SR_SHIFTED_RESIDUAL ? round_to<T>(__ldg(res_shift + ch)) : 0.f;
       for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < row_len; j += gridDim.x * blockDim.x)
-        out[row + j] = from_f<T>(shift_relu1<T, FORM>(to_f(conv[row + j]), s, FORM != SR_PLAIN ? to_f(res[row + j]) : 0.f, t));
+        out[row + j] = from_f<T>(shift_relu1<T, FORM, RELU>(to_f(conv[row + j]), s, FORM != SR_PLAIN ? to_f(res[row + j]) : 0.f, t));
     }
   }
 }
 
 template <typename T, bool NHWC>
-static void launch_shift_relu(int form, dim3 grid, cudaStream_t st, const T* conv, const float* shift, const T* res,
-                              const float* res_shift, T* out, int rows, int row_len, int c) {
-  if (form == SR_PLAIN)
-    shift_relu_kernel<T, NHWC, SR_PLAIN><<<grid, 256, 0, st>>>(conv, shift, res, res_shift, out, rows, row_len, c);
+static void launch_shift_relu(int form, bool relu, dim3 grid, cudaStream_t st, const T* conv, const float* shift,
+                              const T* res, const float* res_shift, T* out, int rows, int row_len, int c) {
+  if (form == SR_PLAIN && !relu)
+    shift_relu_kernel<T, NHWC, SR_PLAIN, false><<<grid, 256, 0, st>>>(conv, shift, res, res_shift, out, rows, row_len, c);
+  else if (form == SR_PLAIN)
+    shift_relu_kernel<T, NHWC, SR_PLAIN, true><<<grid, 256, 0, st>>>(conv, shift, res, res_shift, out, rows, row_len, c);
   else if (form == SR_RESIDUAL)
-    shift_relu_kernel<T, NHWC, SR_RESIDUAL><<<grid, 256, 0, st>>>(conv, shift, res, res_shift, out, rows, row_len, c);
+    shift_relu_kernel<T, NHWC, SR_RESIDUAL, true><<<grid, 256, 0, st>>>(conv, shift, res, res_shift, out, rows, row_len,
+                                                                        c);
   else
-    shift_relu_kernel<T, NHWC, SR_SHIFTED_RESIDUAL><<<grid, 256, 0, st>>>(conv, shift, res, res_shift, out, rows,
-                                                                           row_len, c);
+    shift_relu_kernel<T, NHWC, SR_SHIFTED_RESIDUAL, true><<<grid, 256, 0, st>>>(conv, shift, res, res_shift, out, rows,
+                                                                                 row_len, c);
 }
 
 template <typename T>
 static int shift_relu_fwd(const char* fn, const T* conv, const float* shift, const T* res, const float* res_shift,
-                          T* out, int n, int h, int w, int c, int channels_last, dgod_stream_t stream) {
+                          T* out, int n, int h, int w, int c, int channels_last, int relu, dgod_stream_t stream) {
   DGOD_REQUIRE(n >= 0 && h >= 0 && w >= 0 && c >= 0, "%s: negative size", fn);
   if ((long long)n * h * w * c == 0) return DGOD_OK;
   DGOD_REQUIRE(conv && shift && out, "%s: null pointer", fn);
   DGOD_REQUIRE(res || !res_shift, "%s: res_shift given without res", fn);
+  DGOD_REQUIRE(relu || !res, "%s: the residual forms always end in the ReLU", fn);
   const long long rows = channels_last ? (long long)n * h : (long long)n * c;
   DGOD_REQUIRE(rows <= INT32_MAX && (long long)w * c <= INT32_MAX && (long long)h * w <= INT32_MAX,
                "%s: map too large", fn);
@@ -92,10 +97,10 @@ static int shift_relu_fwd(const char* fn, const T* conv, const float* shift, con
     DGOD_REQUIRE(aligned16(conv) && aligned16(shift) && aligned16(res) && aligned16(res_shift) && aligned16(out),
                  "%s: channels_last needs 16-byte aligned pointers", fn);
     const int row_len = w * (c / N);
-    launch_shift_relu<T, true>(form, row_grid(rows, row_len), st, conv, shift, res, res_shift, out, (int)rows, row_len,
+    launch_shift_relu<T, true>(form, relu != 0, row_grid(rows, row_len), st, conv, shift, res, res_shift, out, (int)rows, row_len,
                                c);
   } else {
-    launch_shift_relu<T, false>(form, row_grid(rows, h * w), st, conv, shift, res, res_shift, out, (int)rows, h * w, c);
+    launch_shift_relu<T, false>(form, relu != 0, row_grid(rows, h * w), st, conv, shift, res, res_shift, out, (int)rows, h * w, c);
   }
   DGOD_LAUNCHED();
   return DGOD_OK;
@@ -107,7 +112,13 @@ using namespace dgod;
 
 extern "C" int dgod_shift_relu_fwd(const float* conv, const float* shift, const float* res, const float* res_shift,
                                    float* out, int n, int h, int w, int c, int channels_last, dgod_stream_t stream) {
-  return shift_relu_fwd<float>("dgod_shift_relu_fwd", conv, shift, res, res_shift, out, n, h, w, c, channels_last,
+  return shift_relu_fwd<float>("dgod_shift_relu_fwd", conv, shift, res, res_shift, out, n, h, w, c, channels_last, 1,
+                               stream);
+}
+
+extern "C" int dgod_bias_add_fwd(const float* conv, const float* bias, float* out, int n, int h, int w, int c,
+                                 int channels_last, dgod_stream_t stream) {
+  return shift_relu_fwd<float>("dgod_bias_add_fwd", conv, bias, nullptr, nullptr, out, n, h, w, c, channels_last, 0,
                                stream);
 }
 
@@ -115,5 +126,5 @@ extern "C" int dgod_shift_relu_fwd_bf16(const void* conv, const float* shift, co
                                         void* out, int n, int h, int w, int c, int channels_last, dgod_stream_t stream) {
   return shift_relu_fwd<__nv_bfloat16>("dgod_shift_relu_fwd_bf16", (const __nv_bfloat16*)conv, shift,
                                        (const __nv_bfloat16*)res, res_shift, (__nv_bfloat16*)out, n, h, w, c,
-                                       channels_last, stream);
+                                       channels_last, 1, stream);
 }

@@ -2,7 +2,7 @@
 `fasterrcnn.FastWILDS` (fasterrcnn.py:354-499) whose detection-head hot path runs on the
 sm_100a kernels.
 
-What stays PyTorch/cuDNN (SURVEY.md L-1): image transform, ResNet-50 + FPN, RPN conv head,
+What stays PyTorch/cuDNN (SURVEY.md L-1): image transform, ResNet-50 + FPN convolutions, the RPN head's 3x3 conv,
 TwoMLPHead / FastRCNNPredictor, the loss arithmetic.  What is replaced (SURVEY.md §8a):
   A1-A4  anchors + decode + per-level top-k + clip/filters + batched NMS   -> ops.rpn_proposals
   A5     assign_targets_to_anchors (box_iou + Matcher + labels)            -> ops.match_boxes
@@ -29,7 +29,7 @@ import torch.nn.functional as F
 from torch import Tensor, nn
 from torchvision.models.detection.backbone_utils import resnet_fpn_backbone
 from torchvision.models.detection.faster_rcnn import FastRCNNPredictor
-from torchvision.models.detection.rpn import RPNHead
+from torchvision.models.detection import rpn as tv_rpn
 from torchvision.models.detection.transform import GeneralizedRCNNTransform
 from torchvision.ops.feature_pyramid_network import FeaturePyramidNetwork
 
@@ -132,6 +132,21 @@ class TwoMLPHead(nn.Module):
 
 
 # ------------------------------------------------------------------------------------ RPN
+class RPNHead(tv_rpn.RPNHead):
+    """torchvision's RPNHead (same modules, parameters and state-dict keys) whose bias, ReLU and 1x1 predictors run as
+    `ops.rpn_head`, one native pass over all levels each way, after the 3x3 conv (cuDNN, without its bias).  On CUDA
+    fp32 NHWC maps with autocast off; anything else (CPU, NCHW, bf16 autocast) is torchvision's forward."""
+
+    def forward(self, x: List[Tensor]) -> Tuple[List[Tensor], List[Tensor]]:
+        block = self.conv[0] if len(self.conv) == 1 else None
+        conv = block[0] if block is not None and len(block) == 2 and isinstance(block[1], nn.ReLU) else None
+        if conv is None or not ops.rpn_head_supported(x, conv, self.cls_logits.weight, self.bbox_pred.weight):
+            return super().forward(x)
+        cs = [conv._conv_forward(f, conv.weight, None) for f in x]
+        return ops.rpn_head(cs, conv.bias, self.cls_logits.weight, self.cls_logits.bias, self.bbox_pred.weight,
+                            self.bbox_pred.bias)
+
+
 class RegionProposalNetwork(nn.Module):
     """fasterrcnn.py:90-196 (RegionProposalNetworkWILDS) on the fused kernels."""
 
@@ -343,9 +358,10 @@ class FusedFPN(FeaturePyramidNetwork):
     """torchvision's FeaturePyramidNetwork (TV ops/feature_pyramid_network.py; fasterrcnn.py:317) whose top-down merge
     runs natively on CUDA: the lateral 1x1 convs run without their bias, and `ops.fpn_top_down` adds the bias, the
     nearest-upsampled coarser level and the lateral in one pass per level (one pass per level backward as well),
-    instead of a bias-add pass, a full-size upsampled copy and an add.  The coarsest lateral conv, the 3x3 layer
-    blocks and LastLevelMaxPool are the stock modules.  Same parameters, state-dict keys and results, bit for bit.  On
-    CPU it is torchvision's forward."""
+    instead of a bias-add pass, a full-size upsampled copy and an add.  The 3x3 layer blocks run their conv without the
+    bias and `ops.bias_add` adds it (under autocast they are the stock modules).  The coarsest lateral conv and
+    LastLevelMaxPool are the stock modules.  Same parameters, state-dict keys and results, bit for bit.  On CPU it is
+    torchvision's forward."""
 
     def forward(self, x: Dict[str, Tensor]) -> Dict[str, Tensor]:
         names, feats = list(x.keys()), list(x.values())
@@ -362,22 +378,26 @@ class FusedFPN(FeaturePyramidNetwork):
             no_bias = [torch.full((conv.out_channels,), -0.0, device=top.device) for conv in convs[:-1]]
             inners = ops.fpn_top_down(laterals, no_bias, top.float())
             inners[-1] = top
+            results = [blk(t) for blk, t in zip(self.layer_blocks, inners)]
         else:
             laterals = [conv._conv_forward(f, conv.weight, None) for conv, f in zip(convs[:-1], feats[:-1])]
             inners = ops.fpn_top_down(laterals, [conv.bias for conv in convs[:-1]], top)
-        results = [blk(t) for blk, t in zip(self.layer_blocks, inners)]
+            # each 3x3 layer block as ATen runs a cuDNN conv: the conv without its bias, then the bias add (natively)
+            layers = [blk[0] for blk in self.layer_blocks]
+            results = [ops.bias_add(conv._conv_forward(t, conv.weight, None), conv.bias) for conv, t in zip(layers, inners)]
         if self.extra_blocks is not None:
             results, names = self.extra_blocks(results, feats, names)
         return OrderedDict(zip(names, results))
 
 
 def fuse_fpn(fpn: FeaturePyramidNetwork) -> None:
-    """Rebinds a stock FeaturePyramidNetwork without norm layers (each inner block a single biased Conv2d) to FusedFPN."""
+    """Rebinds a stock FeaturePyramidNetwork without norm layers (each inner and layer block a single biased Conv2d) to
+    FusedFPN."""
     if type(fpn) is not FeaturePyramidNetwork:
         raise TypeError(f"fuse_fpn expects a torchvision FeaturePyramidNetwork, got {type(fpn).__name__}")
-    for blk in fpn.inner_blocks:
+    for blk in (*fpn.inner_blocks, *fpn.layer_blocks):
         if len(blk) != 1 or type(blk[0]) is not nn.Conv2d or blk[0].bias is None:
-            raise TypeError("fuse_fpn: every inner block must be one Conv2d with a bias (no norm layer)")
+            raise TypeError("fuse_fpn: every inner and layer block must be one Conv2d with a bias (no norm layer)")
     fpn.__class__ = FusedFPN
 
 

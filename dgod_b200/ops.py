@@ -1362,3 +1362,141 @@ def shift_relu(c: Tensor, shift: Tensor, residual: Optional[Tensor] = None, res_
     if res_shift is not None and residual is None:
         raise ValueError("shift_relu: res_shift needs a residual")
     return _ShiftReluFn.apply(c, shift, residual, res_shift)
+
+
+class _BiasAddFn(torch.autograd.Function):
+    """Forward: dgod_bias_add_fwd.  Backward: the gradient itself for the map, and for the bias the
+    sum ATen's convolution_backward takes for a cuDNN convolution's bias, so both stay bit-exact with nn.Conv2d."""
+
+    @staticmethod
+    def forward(ctx, c, bias):
+        c, nhwc = _map_layout(c)
+        bias = _f32c(bias)
+        n, ch, h, w = c.shape
+        if c.dtype != torch.float32 or bias.shape != (ch,):
+            raise RuntimeError(f"bias_add: a float32 map and a ({ch},) bias expected, got {c.dtype} and "
+                               f"{tuple(bias.shape)}")
+        out = torch.empty_like(c)
+        tok = KernelTimer.start("bias_add", 8 * c.numel())
+        check(_lib.load().dgod_bias_add_fwd(_p(c), _p(bias), _p(out), n, h, w, ch, int(nhwc), _stream()))
+        KernelTimer.stop(tok)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        return (g if ctx.needs_input_grad[0] else None), (g.sum((0, 2, 3)) if ctx.needs_input_grad[1] else None)
+
+
+def bias_add(c: Tensor, bias: Tensor) -> Tensor:
+    """c + bias[c] in one pass over an fp32 [N, C, H, W] map (dgod_bias_add_fwd, the shift_relu pass without the ReLU): a biased
+    convolution is conv._conv_forward(x, w, None) followed by this, bit-exact with nn.Conv2d forward and backward.  The
+    result has c's memory layout."""
+    _need_cuda(c, bias)
+    return _BiasAddFn.apply(c, bias)
+
+
+# --------------------------------------------------------------------------------- RPN head after its 3x3 conv
+RPN_HEAD_CHANNELS, RPN_HEAD_ANCHORS = 256, 3
+
+
+def _rpn_head_check(cs: Sequence[Tensor], bias: Tensor, w_cls: Tensor, b_cls: Tensor, w_bbox: Tensor,
+                    b_bbox: Tensor) -> None:
+    C, A = RPN_HEAD_CHANNELS, RPN_HEAD_ANCHORS
+    if not 1 <= len(cs) <= _lib.MAX_LEVELS:
+        raise ValueError(f"rpn_head: 1..{_lib.MAX_LEVELS} levels expected, got {len(cs)}")
+    for i, c in enumerate(cs):
+        if c.dtype != torch.float32 or c.dim() != 4 or c.shape[1] != C or c.shape[0] != cs[0].shape[0]:
+            raise ValueError(f"rpn_head: level {i}: float32 [N, {C}, H, W] maps of one batch expected, got {c.dtype} "
+                             f"{tuple(c.shape)}")
+        if not c.is_contiguous(memory_format=torch.channels_last):
+            raise ValueError(f"rpn_head: level {i}: the map must be channels_last (NHWC)")
+    for name, t, shape in (("bias", bias, (C,)), ("w_cls", w_cls, (A, C, 1, 1)), ("b_cls", b_cls, (A,)),
+                           ("w_bbox", w_bbox, (4 * A, C, 1, 1)), ("b_bbox", b_bbox, (4 * A,))):
+        if t.dtype != torch.float32 or tuple(t.shape) != shape:
+            raise ValueError(f"rpn_head: {name} must be float32 of shape {shape}, got {t.dtype} {tuple(t.shape)}")
+
+
+def _rpn_levels(cs: Sequence[Tensor]):
+    k = len(cs)
+    return (C.c_void_p * k)(*[c.data_ptr() for c in cs]), (C.c_int * k)(*[c.shape[2] for c in cs]), \
+        (C.c_int * k)(*[c.shape[3] for c in cs])
+
+
+def _rpn_head_fwd(cs: Sequence[Tensor], bias: Tensor, w_cls: Tensor, b_cls: Tensor, w_bbox: Tensor, b_bbox: Tensor):
+    A, k = RPN_HEAD_ANCHORS, len(cs)
+    n = cs[0].shape[0]
+    obj = [torch.empty((n, A, c.shape[2], c.shape[3]), dtype=torch.float32, device=c.device) for c in cs]
+    dl = [torch.empty((n, 4 * A, c.shape[2], c.shape[3]), dtype=torch.float32, device=c.device) for c in cs]
+    cp, hs, ws = _rpn_levels(cs)
+    tok = KernelTimer.start("rpn_head_fwd", sum(4 * c.numel() + 4 * 5 * A * c[:, 0].numel() for c in cs))
+    check(_lib.load().dgod_rpn_head_fwd(cp, k, hs, ws, n, RPN_HEAD_CHANNELS, A, _p(bias), _p(w_cls), _p(b_cls),
+                                        _p(w_bbox), _p(b_bbox), (C.c_void_p * k)(*[o.data_ptr() for o in obj]),
+                                        (C.c_void_p * k)(*[d.data_ptr() for d in dl]), _stream()))
+    KernelTimer.stop(tok)
+    return obj, dl
+
+
+def _rpn_head_bwd(cs: Sequence[Tensor], bias: Tensor, w_cls: Tensor, w_bbox: Tensor, g_obj: Sequence[Tensor],
+                  g_dl: Sequence[Tensor]):
+    A, k = RPN_HEAD_ANCHORS, len(cs)
+    lib = _lib.load()
+    gcs = [torch.empty_like(c, memory_format=torch.channels_last) for c in cs]
+    params = torch.empty(RPN_HEAD_CHANNELS * (5 * A + 1) + 5 * A, dtype=torch.float32, device=cs[0].device)
+    ws = _ws(lib.dgod_rpn_head_workspace_bytes(), cs[0].device)
+    cp, hs, wd = _rpn_levels(cs)
+    tok = KernelTimer.start("rpn_head_bwd", sum(8 * c.numel() + 4 * 5 * A * c[:, 0].numel() for c in cs))
+    check(lib.dgod_rpn_head_bwd(cp, k, hs, wd, cs[0].shape[0], RPN_HEAD_CHANNELS, A, _p(bias), _p(w_cls), _p(w_bbox),
+                                (C.c_void_p * k)(*[g.data_ptr() for g in g_obj]),
+                                (C.c_void_p * k)(*[g.data_ptr() for g in g_dl]),
+                                (C.c_void_p * k)(*[g.data_ptr() for g in gcs]), _p(params), _p(ws), ws.numel(),
+                                _stream()))
+    KernelTimer.stop(tok)
+    return gcs, params
+
+
+class _RpnHeadFn(torch.autograd.Function):
+    """The RPN head after its 3x3 conv over all levels: forward dgod_rpn_head_fwd, backward dgod_rpn_head_bwd.  Saves
+    the bias-free conv outputs (the backward recomputes relu(c + bias) from them) instead of the activations."""
+
+    @staticmethod
+    def forward(ctx, bias, w_cls, b_cls, w_bbox, b_bbox, *cs):
+        obj, dl = _rpn_head_fwd(cs, bias, w_cls, b_cls, w_bbox, b_bbox)
+        ctx.save_for_backward(bias, w_cls, w_bbox, *cs)
+        return (*obj, *dl)
+
+    @staticmethod
+    def backward(ctx, *grads):
+        bias, w_cls, w_bbox, *cs = ctx.saved_tensors
+        k, A, Cn = len(cs), RPN_HEAD_ANCHORS, RPN_HEAD_CHANNELS
+        gcs, p = _rpn_head_bwd(cs, bias, w_cls, w_bbox, [_f32c(g) for g in grads[:k]], [_f32c(g) for g in grads[k:]])
+        o1, o2, o3 = A * Cn, 5 * A * Cn, 5 * A * Cn + Cn
+        return (p[o2:o3], p[:o1].view(A, Cn, 1, 1), p[o3:o3 + A], p[o1:o2].view(4 * A, Cn, 1, 1), p[o3 + A:], *gcs)
+
+
+def rpn_head(cs: Sequence[Tensor], bias: Tensor, w_cls: Tensor, b_cls: Tensor, w_bbox: Tensor, b_bbox: Tensor):
+    """torchvision's RPNHead forward after its 3x3 conv, all levels in one launch each way: `cs` are the conv's outputs
+    WITHOUT its bias (conv._conv_forward(x, w, None)), fp32 NHWC [N, 256, H, W]; `bias` the conv's bias; w_cls / b_cls
+    and w_bbox / b_bbox the cls_logits and bbox_pred 1x1 convs' parameters (3 anchors per location).  Returns
+    (objectness, deltas): lists of NCHW-contiguous [N, 3, H, W] / [N, 12, H, W].  The 1x1 products are fp32 fma chains
+    (not TF32); relu(c + bias) is bit-identical to the stock conv + relu_."""
+    cs = list(cs)
+    _rpn_head_check(cs, bias, w_cls, b_cls, w_bbox, b_bbox)
+    _need_cuda(*cs, bias, w_cls, b_cls, w_bbox, b_bbox)
+    params = tuple(t.contiguous() for t in (bias, w_cls, b_cls, w_bbox, b_bbox))
+    k = len(cs)
+    if torch.is_grad_enabled() and any(t.requires_grad for t in (*cs, *params)):
+        out = _RpnHeadFn.apply(*params, *cs)
+        return list(out[:k]), list(out[k:])
+    return _rpn_head_fwd(cs, *params)
+
+
+def rpn_head_supported(feats: Sequence[Tensor], conv: "torch.nn.Conv2d", w_cls: Tensor, w_bbox: Tensor) -> bool:
+    """Whether RPNHead's forward can run on rpn_head: CUDA fp32 NHWC maps of 256 channels, autocast off, a 3x3 conv
+    with a bias, 3 anchors per location, fp32 parameters 16-byte aligned."""
+    params = (conv.weight, conv.bias, w_cls, w_bbox)
+    return (len(feats) >= 1 and len(feats) <= _lib.MAX_LEVELS and not torch.is_autocast_enabled("cuda")
+            and conv.bias is not None and conv.out_channels == RPN_HEAD_CHANNELS
+            and w_cls.shape[0] == RPN_HEAD_ANCHORS
+            and all(p.is_cuda and p.dtype == torch.float32 and p.data_ptr() % 16 == 0 for p in params)
+            and all(f.is_cuda and f.dtype == torch.float32 and f.dim() == 4 and f.shape[0] == feats[0].shape[0]
+                    and f.is_contiguous(memory_format=torch.channels_last) for f in feats))

@@ -36,6 +36,7 @@
  *                           upsample, add) and its autograd (upsample_nearest2d_backward + accumulation)
  *   dgod_stem_pool_fwd      TV models/resnet.py ResNet._forward_impl: bn1 shift (folded), relu, maxpool of a frozen stem
  *   dgod_shift_relu_fwd     TV models/resnet.py Bottleneck.forward: bn1-3 and downsample shifts (folded), residual add, relu
+ *   dgod_bias_add_fwd       the bias add of a cuDNN convolution: TV ops/feature_pyramid_network.py FPN layer blocks
  *   dgod_*_bf16             the four backbone entry points above on bf16 maps: the same modules under
  *                           torch.autocast("cuda", dtype=torch.bfloat16)
  *   dgod_map_match          torchmetrics MeanAveragePrecision (pycocotools backend): COCOeval.computeIoU / evaluateImg,
@@ -43,6 +44,8 @@
  *   dgod_map_accumulate     the same: COCOeval.accumulate
  *   dgod_linear_tc          TV models/detection/faster_rcnn.py TwoMLPHead (fasterrcnn.py:331-352): fc6 / fc7 Linear
  *                           forward (bias, ReLU) and their autograd products, fp32-accurate on the tensor cores
+ *   dgod_rpn_head_fwd/_bwd  TV models/detection/rpn.py RPNHead.forward after its 3x3 conv (fasterrcnn.py:165): bias, relu,
+ *                           the two 1x1 predictors, and their autograd (dgrads, threshold_backward, weight / bias grads)
  */
 #ifndef DGOD_B200_H_
 #define DGOD_B200_H_
@@ -56,7 +59,7 @@ extern "C" {
 
 typedef void* dgod_stream_t; /* a cudaStream_t (0 = legacy default stream) */
 
-#define DGOD_ABI_VERSION 8
+#define DGOD_ABI_VERSION 9
 
 enum {
   DGOD_OK = 0,
@@ -386,6 +389,9 @@ int dgod_stem_pool_fwd(const float* conv, const float* shift /*device [c]*/, flo
 int dgod_shift_relu_fwd(const float* conv, const float* shift /*device [c]*/, const float* res,
                         const float* res_shift /*device [c]*/, float* out, int n, int h, int w, int c, int channels_last,
                         dgod_stream_t stream);
+/* The same pass without the ReLU: out = conv + bias[c], a convolution's bias add, bit-exact with ATen's add_. */
+int dgod_bias_add_fwd(const float* conv, const float* bias /*device [c]*/, float* out, int n, int h, int w, int c,
+                      int channels_last, dgod_stream_t stream);
 
 /* The same four on bf16 maps (__nv_bfloat16 [n, c, h, w]; channels_last needs c % 8 == 0 and 16-byte aligned pointers);
  * biases and shifts stay fp32.  Bit-exact with the ATen bf16 ops under autocast: fp32 math, every add's result rounded
@@ -443,6 +449,29 @@ int dgod_map_accumulate(const uint32_t* tp_mask, const int* seg_offsets, const i
 size_t dgod_linear_tc_workspace_bytes(int m, int n, int k);
 int dgod_linear_tc(const float* a, int a_trans, const float* b, int b_trans, int m, int n, int k, const float* bias,
                    int relu, const float* mask, float* c, void* workspace, size_t workspace_bytes, dgod_stream_t stream);
+
+/* ------------------------------------------------------------------ RPN head (after its 3x3 conv) */
+
+/* All n_levels (<= DGOD_MAX_LEVELS) levels in one launch.  c[l]: the 3x3 conv's output WITHOUT its bias, NHWC fp32
+ * [n_img, height[l], width[l], channels] (16-byte aligned); channels == 256 and anchors == 3 only.  bias [channels]
+ * (the 3x3 conv's), w_cls [anchors, channels], b_cls [anchors], w_bbox [4 anchors, channels], b_bbox [4 anchors]:
+ * device fp32, weights and bias 16-byte aligned.  With t = relu_(c + bias) (clamp_min: NaN passes):
+ * objectness[l] [n_img, anchors, h, w] = W_cls t + b_cls and deltas[l] [n_img, 4 anchors, h, w] = W_bbox t + b_bbox,
+ * NCHW-contiguous, each product an fp32 fma chain over the channels in ascending order. */
+int dgod_rpn_head_fwd(const float* const* c, int n_levels, const int* height, const int* width, int n_img, int channels,
+                      int anchors, const float* bias, const float* w_cls, const float* b_cls, const float* w_bbox,
+                      const float* b_bbox, float* const* objectness, float* const* deltas, dgod_stream_t stream);
+/* Its backward from the incoming gradients grad_objectness[l] / grad_deltas[l] (NCHW-contiguous, shapes of the
+ * outputs above): grad_c[l] (NHWC like c) = (t <= 0) ? 0 : W_cls^T g_obj + W_bbox^T g_deltas (threshold_backward), and
+ * grad_params [256 * 15 + 256 + 15] = dW_cls [3, 256], dW_bbox [12, 256], d bias [256], d b_cls [3], d b_bbox [12],
+ * each summed over every pixel of every level.  Deterministic (fixed partition and summation order, no atomics).  Two
+ * launches, the second a programmatic dependent launch.  Workspace: dgod_rpn_head_workspace_bytes() (depends on the
+ * current device's SM count; 0 if it cannot be queried). */
+size_t dgod_rpn_head_workspace_bytes(void);
+int dgod_rpn_head_bwd(const float* const* c, int n_levels, const int* height, const int* width, int n_img, int channels,
+                      int anchors, const float* bias, const float* w_cls, const float* w_bbox,
+                      const float* const* grad_objectness, const float* const* grad_deltas, float* const* grad_c,
+                      float* grad_params, void* workspace, size_t workspace_bytes, dgod_stream_t stream);
 
 /* ------------------------------------------------------------------ gradient reversal */
 
